@@ -75,6 +75,8 @@ def parse_args():
                     "(oracle/_ref/libmm_ref.so: its own index build from FASTA, its own mapModule); 'port' = the oracle restatement on the "
                     "product's index content; 'auto' = real when the library is there")
     ap.add_argument("--as-rank", type=int, default=-1, help="debug: generate the reads rank R of a multi-GPU run would get (read seed 2 + R)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="after the timed steps, write what the last step computed as "
+                    "DIR/<name>.npy (float64; a fixed, seeded sample of the fragments and reads), see dump_outputs()")
     return ap.parse_args()
 
 
@@ -543,6 +545,8 @@ def gpu_arm(args):
 
     # ---- correctness of what was timed ----
     res = bm.results()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, seg_res, cands, loci, res, wl["first_counter"], n_local)
     acc = _accuracy(res, wl["truth"], wl["contig_len"], wl["first_counter"], wl["lo"]) if wl["truth"] is not None else None
     sharded_check = None
     if strong and world > 1 and rank == 0 and one_to_one:
@@ -641,6 +645,55 @@ def gpu_arm(args):
         if comm is not None:
             comm.close()
         dist.destroy_process_group()
+
+
+DUMP_SEGMENTS = 65_536  # fragments sampled for --dump-outputs (of 2 M at the default size): ~14 MB of .npy in all
+DUMP_READS = 32_768
+
+
+def _ranges(first, count):
+    """indices first[i] .. first[i] + count[i] - 1 of every i, concatenated, and the i each one belongs to"""
+    count = count.astype(np.int64)
+    owner = np.repeat(np.arange(len(count)), count)
+    starts = np.repeat(first.astype(np.int64) - np.concatenate([[0], np.cumsum(count)[:-1]]), count)
+    return starts + np.arange(int(count.sum())), owner
+
+
+def dump_outputs(out_dir, seg_res, cands, loci, res, first_counter, n_reads):
+    """What the last timed step handed its caller, as float64 .npy files that two builds can be compared on:
+      segments.npy    value path (mm_map_resident), per sampled fragment: fragment index, sketch_max_hash >> 32,
+                      sketch_max_hash & 0xffffffff, sketch_raw_count, sketch_size, n_points, minimum_hits, best_intersection,
+                      n_candidates
+      candidates.npy  the L1 candidates of those fragments in fragment order: fragment index, seqId, rangeStartPos, rangeEndPos,
+                      intersectionSize, n_loci
+      loci.npy        their L2 loci in the same order: fragment index, seqId, meanOptimalPos, optimalStart, optimalEnd,
+                      sharedSketchSize, strand
+      mappings.npy    e2e path (skch::BatchMapper): the mapping rows of a sample of the reads, as results() returns them
+    The fragments' first_candidate / first_locus offsets are left out: they depend on the order the CTAs reserved their
+    slices in, not on what was computed. The samples are drawn with a fixed seed from the fragment / read counts only."""
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(12345)
+    n = len(seg_res)
+    pick = np.sort(rng.choice(n, min(n, DUMP_SEGMENTS), replace=False))
+    sr = seg_res[pick]
+    h = sr["sketch_max_hash"]
+    np.save(os.path.join(out_dir, "segments.npy"), np.stack(
+        [pick, h >> np.uint64(32), h & np.uint64(0xFFFFFFFF)] + [sr[f] for f in ("sketch_raw_count", "sketch_size", "n_points",
+                                                                                  "minimum_hits", "best_intersection", "n_candidates")],
+        axis=1).astype(np.float64))
+    ci, owner = _ranges(sr["first_candidate"], sr["n_candidates"])
+    c = cands[ci]
+    np.save(os.path.join(out_dir, "candidates.npy"), np.stack(
+        [pick[owner]] + [c[f] for f in ("seqId", "rangeStartPos", "rangeEndPos", "intersectionSize", "n_loci")], axis=1).astype(np.float64))
+    li, lowner = _ranges(c["first_locus"], c["n_loci"])
+    lc = loci[li]
+    np.save(os.path.join(out_dir, "loci.npy"), np.stack(
+        [pick[owner[lowner]]] + [lc[f] for f in ("seqId", "meanOptimalPos", "optimalStart", "optimalEnd", "sharedSketchSize", "strand")],
+        axis=1).astype(np.float64))
+    keep = np.sort(rng.choice(n_reads, min(n_reads, DUMP_READS), replace=False)) + first_counter
+    np.save(os.path.join(out_dir, "mappings.npy"), res[np.isin(res[:, 0], keep)].astype(np.float64))
+    log(f"outputs of the last step written to {out_dir}: {len(pick)} fragments, {len(c)} candidates, {len(lc)} loci, "
+        f"mappings of {len(keep)} reads")
 
 
 def algorithmic_bytes_l1_l2(seg_res, cands, loci, idx_seq, idx_wpos, seg_len):

@@ -1,6 +1,9 @@
 """The product's option parser fills skch::Parameters exactly as the reference's parseandSave does
 (reference src/map/include/parseCmdArgs.hpp:257-659: defaults, automatic sketch size from the file size, --dense,
-filter modes, chaining / block-length defaults, skip-self when no query is given ...). CPU only."""
+filter modes, chaining / block-length defaults, skip-self when no query is given ...). CPU only. The reference's
+Parameters for every command line here are stored in tests/golden/reference_params.json (written by
+tests/golden/make_reference_params.py through oracle/_ref), so the comparison needs no reference build."""
+import json
 import os
 
 import pytest
@@ -9,7 +12,7 @@ import datasets
 import refh
 from mashmap_b200 import hostlib
 
-pytestmark = pytest.mark.skipif(not refh.available(), reason="oracle/_ref not built")
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_params.json")
 
 OPTION_SETS = [
     [],
@@ -31,35 +34,56 @@ def d(workdir):
     return datasets.make_panel_set(workdir, tag="args", n_strains=2, chrom_len=40_000)
 
 
+def cli_args(d, opts, with_query):
+    return ["-r", d["ref"]] + (["-q", d["qry"]] if with_query else []) + ["-t", "2"] + opts
+
+
+def params_key(opts, with_query):
+    return " ".join(["with query" if with_query else "no query"] + opts)
+
+
+def size_args(path):
+    return ["-r", path, "-q", path, "-s", "5000", "--pi", "85"]
+
+
+def write_sparse_fasta(path, size):
+    with open(path, "wb") as fh:
+        fh.write(b">c\nACGT\n")
+        fh.truncate(size)
+
+
+def reference_params(key):
+    """skch::Parameters the reference's parseandSave filled for the command line `key`, as {field: value}"""
+    with open(GOLDEN) as f:
+        return json.load(f)[key]
+
+
 @pytest.mark.parametrize("opts", OPTION_SETS, ids=lambda o: " ".join(o) or "defaults")
 @pytest.mark.parametrize("with_query", [True, False])
 def test_parameters_equal_reference(d, opts, with_query):
-    args = ["-r", d["ref"]] + (["-q", d["qry"]] if with_query else []) + ["-t", "2"] + opts
-    R = refh.RefSession(args)
-    try:
-        ours = hostlib.HostIndex.from_cli(args)
-        p = ours.params_into(refh.OrcParams())
-        for name, _ in refh.OrcParams._fields_:
-            a, b = getattr(R.p, name), getattr(p, name)
-            assert a == b, (name, a, b, args)
-        ours.close()
-    finally:
-        R.close()
+    args = cli_args(d, opts, with_query)
+    ref = reference_params(params_key(opts, with_query))
+    ours = hostlib.HostIndex.from_cli(args)
+    p = ours.params_into(refh.OrcParams())
+    for name, _ in refh.OrcParams._fields_:
+        a, b = ref[name], getattr(p, name)
+        assert a == b, (name, a, b, args)
+    ours.close()
 
 
-@pytest.mark.parametrize("size", [2**31 - 1000, 2**31 + 1000, 3_100_000_000, 5_000_000_000, 2**32 + 4096])
+SIZES = [2**31 - 1000, 2**31 + 1000, 3_100_000_000, 5_000_000_000, 2**32 + 4096]
+
+
+@pytest.mark.parametrize("size", SIZES)
 def test_reference_size_wraps_like_the_reference(tmp_path, size):
     """map_parameters.hpp:41 keeps referenceSize in an offset_t (int32): for files >= 2 GiB the value wraps and is
     sign-extended into recommendedSketchSize (parseCmdArgs.hpp:304,639), so the automatic sketch size differs from the
     one the formula gives for the true size. The product reproduces that (a sparse file stands in for the FASTA)."""
-    f = tmp_path / "big.fa"
-    with open(f, "wb") as fh:
-        fh.write(b">c\nACGT\n")
-        fh.truncate(size)
-    args = ["-r", str(f), "-q", str(f), "-s", "5000", "--pi", "85"]
-    ref = refh.parse_only(args)
-    ours = hostlib.HostIndex.params_from_cli(args)
+    f = str(tmp_path / "big.fa")
+    write_sparse_fasta(f, size)
+    ref = reference_params(f"size {size}")
+    ours = hostlib.HostIndex.params_from_cli(size_args(f))
     p = ours.params_into(refh.OrcParams())
     ours.close()
-    assert p.referenceSize == ref.referenceSize
-    assert p.sketchSize == ref.sketchSize
+    assert p.referenceSize == ref["referenceSize"]
+    assert p.sketchSize == ref["sketchSize"]

@@ -1,6 +1,10 @@
 """CPU tests of the host-side product code (no GPU): statistics tables, the host index builder and the
-host tail, each against the UNMODIFIED reference through oracle/_ref (when built)."""
+host tail, each against the UNMODIFIED reference through oracle/_ref (when built). The statistics tables of the
+reference are stored in tests/golden/reference_stats.json (written by tests/golden/make_reference_stats.py), so those
+comparisons need no reference build."""
 import ctypes as C
+import json
+import os
 
 import numpy as np
 import pytest
@@ -10,6 +14,43 @@ import refh
 from mashmap_b200 import capi, hostlib, synth
 
 needs_ref = pytest.mark.skipif(not refh.available(), reason="oracle/_ref not built")
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "reference_stats.json")
+MIN_HITS_PI = [0.85, 0.90, 0.95, 0.80]
+MIN_HITS_S = list(range(1, 420)) + [500, 777, 1000]
+STAT_K = (15, 19, 21)
+LOWER_BOUND_S = (20, 130, 220, 400)
+SKETCH_SIZE_CASES = [(size, pi, seg) for size in (1_200_000, 25_711_390, 100_000_000, 3_050_000_000)
+                     for pi, seg in ((0.85, 5000), (0.95, 5000), (0.90, 10000), (0.85, 1000))]
+CUTOFF_ARGS = [["-s", "5000", "--pi", "85"], ["-s", "5000", "--pi", "95", "--dense"], ["-s", "2000", "--pi", "90", "-J", "25"],
+               ["-s", "5000", "--pi", "85", "--hgFilterAniDiff", "2", "--hgFilterConf", "99"]]
+
+
+def reference_stats(key):
+    """the reference's values for one table of this module (see tests/golden/make_reference_stats.py)"""
+    with open(GOLDEN) as f:
+        return json.load(f)[key]
+
+
+def stat_inputs():
+    """the Jaccard values the float functions are compared on"""
+    rng = np.random.default_rng(3)
+    return np.concatenate([rng.random(200).astype(np.float32), np.float32([0, 1, 0.5, 1e-6])])
+
+
+def lower_bound_inputs():
+    """(s, shared) pairs of the mash-distance lower bound"""
+    return [(s, shared) for s in LOWER_BOUND_S for shared in range(0, s + 1, max(1, s // 37))]
+
+
+def f32_bits(x):
+    return int(np.float32(x).view(np.uint32))
+
+
+def write_cutoff_fasta(workdir):
+    ref = os.path.join(workdir, "cut_ref.fa")
+    synth.write_fasta(ref, ["c0"], synth.random_genome(1, 60_000, seed=8))
+    return ref
 
 
 def test_c_abi_library_loads_and_exports_every_symbol():
@@ -53,41 +94,35 @@ def test_no_cpu_fallback_without_device():
     assert e.value.code == capi.MM_ENODEVICE
 
 
-@needs_ref
-@pytest.mark.parametrize("pi", [0.85, 0.90, 0.95, 0.80])
+@pytest.mark.parametrize("pi", MIN_HITS_PI)
 def test_min_hits_table_matches_reference(pi):
-    R = refh.lib()
+    ref = reference_stats(f"min_hits {pi}")
     L = hostlib.lib()
     for k in (19, 16):
-        for s in list(range(1, 420)) + [500, 777, 1000]:
-            assert L.skch_min_hits(s, k, pi) == R.refh_min_hits(s, k, pi), (s, k, pi)
+        for s, want in zip(MIN_HITS_S, ref[str(k)], strict=True):
+            assert L.skch_min_hits(s, k, pi) == want, (s, k, pi)
 
 
-@needs_ref
 def test_float_stat_functions_bit_equal():
-    R = refh.lib()
+    ref = reference_stats("float functions")
     L = hostlib.lib()
-    rng = np.random.default_rng(3)
-    for j in np.concatenate([rng.random(200).astype(np.float32), np.float32([0, 1, 0.5, 1e-6])]):
-        for k in (15, 19, 21):
-            a, b = L.skch_j2md(float(j), k), R.refh_j2md(float(j), k)
-            assert np.float32(a).tobytes() == np.float32(b).tobytes()
-            a, b = L.skch_md2j(float(j), k), R.refh_md2j(float(j), k)
-            assert np.float32(a).tobytes() == np.float32(b).tobytes()
-    for s in (20, 130, 220, 400):
-        for shared in range(0, s + 1, max(1, s // 37)):
-            d = R.refh_j2md(np.float32(shared / s), 19)
-            a, b = L.skch_md_lower_bound(d, s, 19), R.refh_md_lower_bound(d, s, 19)
-            assert np.float32(a).tobytes() == np.float32(b).tobytes(), (s, shared)
+    assert len(ref["j2md"]) == len(ref["md2j"]) == len(stat_inputs()) * len(STAT_K)
+    i = 0
+    for j in stat_inputs():
+        for k in STAT_K:
+            assert f32_bits(L.skch_j2md(float(j), k)) == ref["j2md"][i]
+            assert f32_bits(L.skch_md2j(float(j), k)) == ref["md2j"][i]
+            i += 1
+    for (s, shared), d, want in zip(lower_bound_inputs(), ref["lower_bound_d"], ref["md_lower_bound"], strict=True):
+        d = float(np.uint32(d).view(np.float32))
+        assert f32_bits(L.skch_md_lower_bound(d, s, 19)) == want, (s, shared)
 
 
-@needs_ref
 def test_recommended_sketch_size_matches_reference():
-    R = refh.lib()
+    ref = reference_stats("recommended sketch size")
     L = hostlib.lib()
-    for size in (1_200_000, 25_711_390, 100_000_000, 3_050_000_000):
-        for pi, seg in ((0.85, 5000), (0.95, 5000), (0.90, 10000), (0.85, 1000)):
-            assert L.skch_recommended_sketch_size(19, pi, seg, size) == R.refh_recommended_sketch_size(19, pi, seg, size)
+    for (size, pi, seg), want in zip(SKETCH_SIZE_CASES, ref, strict=True):
+        assert L.skch_recommended_sketch_size(19, pi, seg, size) == want, (size, pi, seg)
 
 
 def test_binomial_tail_against_exact_summation():
@@ -103,21 +138,13 @@ def test_binomial_tail_against_exact_summation():
             assert abs(got - exact) <= 1e-12 + 1e-9 * exact, (n, p, k, got, exact)
 
 
-@needs_ref
-@pytest.mark.parametrize("args", [["-s", "5000", "--pi", "85"], ["-s", "5000", "--pi", "95", "--dense"],
-                                  ["-s", "2000", "--pi", "90", "-J", "25"],
-                                  ["-s", "5000", "--pi", "85", "--hgFilterAniDiff", "2", "--hgFilterConf", "99"]])
-def test_sketch_cutoffs_match_reference(workdir, args):
-    import os
-
-    ref = os.path.join(workdir, "cut_ref.fa")
-    synth.write_fasta(ref, ["c0"], synth.random_genome(1, 60_000, seed=8))
-    R = refh.RefSession(["-r", ref, "-q", ref] + args)
-    try:
-        got = hostlib.sketch_cutoffs(R.p.sketchSize, R.p.kmerSize, R.p.ANIDiff, R.p.ANIDiffConf, bool(R.p.stage1_topANI_filter))
-        assert np.array_equal(got, R.cutoffs())
-    finally:
-        R.close()
+@pytest.mark.parametrize("args", CUTOFF_ARGS)
+def test_sketch_cutoffs_match_reference(args):
+    """the cut-off table for the reference's own Parameters of a 60 kb reference file"""
+    ref = reference_stats("cutoffs " + " ".join(args))
+    p = ref["params"]
+    got = hostlib.sketch_cutoffs(p["sketchSize"], p["kmerSize"], p["ANIDiff"], p["ANIDiffConf"], bool(p["stage1_topANI_filter"]))
+    assert np.array_equal(got, ref["value"])
 
 
 def _cases_for_index():
