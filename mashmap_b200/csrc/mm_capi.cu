@@ -7,7 +7,6 @@
  * fails with MM_ENODEVICE.
  */
 #include <algorithm>
-#include <atomic>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -20,6 +19,57 @@
 #include <chrono>
 
 static thread_local std::string g_create_error;
+
+namespace {
+
+int fail(mm_ctx *c, int code, const char *fmt, ...);
+
+/* A device array that frees itself: the context's batch buffers and the temporaries of the index builders. */
+template <typename T>
+struct dev_array {
+  T *p = nullptr;
+  uint64_t cap = 0; /* elements */
+  dev_array() = default;
+  dev_array(const dev_array &) = delete;
+  dev_array &operator=(const dev_array &) = delete;
+  ~dev_array() { release(); }
+  void release() { cudaFree(p); p = nullptr; cap = 0; }
+  /* room for `need` elements: kept if it has them, else replaced (contents lost) by `new_cap` elements, *fresh = true.
+   * The capacity changes only once the allocation has succeeded, and a failed one is not left as the last error. */
+  int reserve(mm_ctx *c, uint64_t need, uint64_t new_cap, bool *fresh = nullptr)
+  {
+    if (fresh) *fresh = false;
+    if (p && need <= cap) return MM_OK;
+    release();
+    const cudaError_t e = cudaMalloc((void **)&p, new_cap * sizeof(T));
+    if (e != cudaSuccess) {
+      p = nullptr;
+      cudaGetLastError();
+      return fail(c, e == cudaErrorMemoryAllocation ? MM_ENOMEM : MM_ECUDA, "cannot allocate %llu bytes of device memory: %s",
+                  (unsigned long long)(new_cap * sizeof(T)), cudaGetErrorString(e));
+    }
+    cap = new_cap;
+    if (fresh) *fresh = true;
+    return MM_OK;
+  }
+};
+
+/* the context's timing events (mm_last_stage_ms, mm_last_pack_ms); EV_BEGIN is in front of K0 (pack) / K1, EV_PREP_* around
+ * the L2 record-preparation kernel */
+enum stage_event { EV_BEGIN, EV_K1_BEGIN, EV_K1_END, EV_K2_END, EV_K3_BEGIN, EV_K3_END, EV_PREP_BEGIN, EV_PREP_END,
+                   EV_H2D_BEGIN, EV_H2D_END, EV_D2H_BEGIN, EV_D2H_END, EV_COUNT };
+struct event_set {
+  cudaEvent_t ev[EV_COUNT] = {};
+  event_set() = default;
+  event_set(const event_set &) = delete;
+  event_set &operator=(const event_set &) = delete;
+  ~event_set() { for (cudaEvent_t e : ev) if (e) cudaEventDestroy(e); }
+  cudaEvent_t operator[](stage_event i) const { return ev[i]; }
+};
+
+constexpr uint32_t L2_LOCI_PER_CAND = 2; /* fixed locus slots per candidate of the stream kernels; more -> general kernel */
+
+} // namespace
 
 struct mm_ctx {
   int device = -1;
@@ -40,40 +90,41 @@ struct mm_ctx {
   std::vector<int32_t> cutoffs, min_hits;
 
   /* batch */
-  uint8_t *d_bases = nullptr; uint64_t bases_cap = 0; uint64_t n_bases = 0;
-  uint8_t *d_packed = nullptr; uint64_t packed_cap = 0; /* nibbles, bytes */
+  dev_array<uint8_t> d_bases; uint64_t n_bases = 0;
+  dev_array<uint8_t> d_packed; /* nibbles */
   mm_built_index built{}; /* lookup arrays of an index built on the device, kept for mm_index_download (keep_lookup) */
   bool built_kept = false;
   bool batch_is_ascii = false; /* the resident batch came in as text: K0 (pack) runs in front of K1 */
-  cudaEvent_t ev_pack = nullptr;
   float pack_ms = 0;
-  mm_segment *d_segs = nullptr; uint64_t segs_cap = 0; uint64_t n_segs = 0;
-  uint64_t *d_sk_hash = nullptr; uint64_t *d_sk_val = nullptr; int2 *d_sk_pos = nullptr; int8_t *d_sk_strand = nullptr; uint64_t sk_cap = 0;
-  mm_segment_result *d_seg_res = nullptr;
-  uint32_t *d_sk_reject = nullptr;
+  dev_array<mm_segment> d_segs; uint64_t n_segs = 0;
+  dev_array<uint64_t> d_sk_hash, d_sk_val; dev_array<int2> d_sk_pos; dev_array<int8_t> d_sk_strand;
+  dev_array<mm_segment_result> d_seg_res;
+  dev_array<uint32_t> d_sk_reject;
   int sk_mode = 0; /* 0 = fast sketch kernel + general kernel over its rejects; 1 = general kernel only (MM_SKETCH_TABLE=1) */
-  mm_l1_candidate *d_cands = nullptr; uint64_t cand_cap = 0;
-  mm_l2_locus *d_loci = nullptr; uint64_t loci_cap = 0;
-  uint32_t *d_counters = nullptr;
+  dev_array<mm_l1_candidate> d_cands;
+  dev_array<mm_l2_locus> d_loci;
+  dev_array<uint32_t> d_counters;
   bool blocking_wait = false;       /* MM_BLOCKING_WAIT=1: host waits block on an event instead of spinning (experiment) */
   cudaEvent_t ev_wait = nullptr;
   const mm_ctx *share_src = nullptr; /* mm_ctx_share_index: the context whose index image this one reads */
   mm_phase_hook hook = nullptr;
   void *hook_user = nullptr;
   uint32_t *h_pub = nullptr; /* pinned, device-mapped: kernels publish counters here (no copy engine involved) */
-  uint64_t *d_scratch = nullptr; uint64_t scratch_cap = 0; uint64_t scratch_slice = 0; uint64_t scratch_pool = 0;
+  dev_array<uint64_t> d_scratch; uint64_t scratch_slice = 0; uint64_t scratch_pool = 0;
+  uint64_t l1_pool0 = 32ULL << 20; /* interval points the bump pool holds at first (grown on demand; MM_L1_POOL_ELEMS) */
   uint32_t l1_grid = 0;
   uint64_t n_cands = 0, n_loci = 0;
-  mm_l2_range *d_l2_ranges = nullptr; uint64_t *d_l2_rec_off = nullptr; uint64_t l2_cand_cap = 0;
-  uint2 *d_l2_recs = nullptr; uint64_t l2_recs_cap = 0;
-  void *d_scan_tmp = nullptr; size_t scan_tmp_bytes = 0;
-  uint32_t *d_l1_slow = nullptr; uint64_t l1_slow_cap = 0;
-  void *d_l2_order = nullptr; size_t l2_order_bytes = 0; /* work area of the candidate ordering (mm_launch_l2_order) */
+  /* per-candidate L2 work areas, grown together: l2_cand_cap is recorded once all four are allocated */
+  dev_array<mm_l2_range> d_l2_ranges; dev_array<uint64_t> d_l2_rec_off; uint64_t l2_cand_cap = 0;
+  dev_array<uint8_t> d_scan_tmp;
+  dev_array<uint8_t> d_l2_order; /* work area of the candidate ordering (mm_launch_l2_order) */
+  dev_array<uint2> d_l2_recs;
+  dev_array<uint32_t> d_l1_slow;
   int l1_warp = 1; /* 1 = warp-per-segment fast path + CTA path for big segments; 0 = CTA path only (MM_L1_CTA=1) */
   int l2_mode = 1; /* 1 = stream kernels (mm_l2_stream.cu), 0 = general kernel only (MM_L2_GENERAL=1) */
   bool batch_mapped = false;
 
-  cudaEvent_t ev[10]{};
+  event_set ev;
   float stage_ms[8]{};
 };
 
@@ -97,17 +148,6 @@ int fail(mm_ctx *c, int code, const char *fmt, ...)
       return fail(c, e_ == cudaErrorMemoryAllocation ? MM_ENOMEM : MM_ECUDA, "%s: %s", #call,    \
                   cudaGetErrorString(e_));                                                       \
   } while (0)
-
-template <typename T>
-int grow(mm_ctx *c, T *&ptr, uint64_t &cap, uint64_t need, uint64_t pad = 0)
-{
-  if (need + pad <= cap && ptr) return MM_OK;
-  if (ptr) { cudaFree(ptr); ptr = nullptr; cap = 0; }
-  uint64_t n = need + pad;
-  CU(c, cudaMalloc((void **)&ptr, n * sizeof(T)));
-  cap = n;
-  return MM_OK;
-}
 
 uint64_t align_up(uint64_t x, uint64_t a) { return (x + a - 1) / a * a; }
 
@@ -154,6 +194,82 @@ int write_tables(mm_ctx *c)
   return MM_OK;
 }
 
+/* The index image's layout (mm_internal.h): the header, then each region at the next 256-byte boundary. */
+mm_blob_header blob_layout(uint64_t n_minmers, uint64_t n_keys, uint64_t n_points, int32_t n_contigs)
+{
+  mm_blob_header h{};
+  h.magic = MM_BLOB_MAGIC;
+  h.n_minmers = n_minmers; h.n_keys = n_keys; h.n_points = n_points;
+  h.n_contigs = n_contigs;
+  h.tab_log2 = 4;
+  while ((1ULL << h.tab_log2) < 2 * n_keys + 2) h.tab_log2++;
+  uint64_t o = align_up(sizeof(mm_blob_header), 256);
+  auto place = [&](uint64_t bytes) { uint64_t at = o; o = align_up(o + bytes, 256); return at; };
+  h.off_idx_hash = place((n_minmers + 1) * 8);
+  h.off_idx_wpos = place((n_minmers + 1) * 4);
+  h.off_idx_wend = place((n_minmers + 1) * 4);
+  h.off_idx_strand = place(n_minmers + 1);
+  h.off_contig_start = place(((uint64_t)n_contigs + 1) * 8);
+  h.off_idx2_hash = place((n_minmers + 1) * 8);
+  h.off_idx2_wend = place((n_minmers + 1) * 4);
+  h.off_tab = place((1ULL << h.tab_log2) * sizeof(mm_tab_slot));
+  h.off_pts = place((n_points + 1) * 8);
+  h.off_contig_len = place((uint64_t)n_contigs * 4);
+  h.off_contig_name_id = place((uint64_t)n_contigs * 4);
+  h.off_contig_group = place((uint64_t)n_contigs * 4);
+  h.off_cutoffs = place(TABLE_REGION_BYTES);
+  h.off_min_hits = place(TABLE_REGION_BYTES);
+  h.total_bytes = o;
+  return h;
+}
+
+/* the context no longer has an index image; it is freed if the context owns it */
+void release_blob(mm_ctx *c)
+{
+  if (c->blob && c->blob_owned) { cudaSetDevice(c->device); cudaFree(c->blob); }
+  c->blob = nullptr; c->blob_bytes = 0; c->blob_ready = false;
+}
+
+/* a new index image of h.total_bytes bytes, owned by the context, in place of the old one; it is not ready until
+ * finish_blob, and a blob_guard frees it on every return before that */
+int replace_blob(mm_ctx *c, const mm_blob_header &h)
+{
+  release_blob(c);
+  const cudaError_t e = cudaMalloc((void **)&c->blob, h.total_bytes);
+  if (e != cudaSuccess) {
+    c->blob = nullptr;
+    cudaGetLastError();
+    return fail(c, e == cudaErrorMemoryAllocation ? MM_ENOMEM : MM_ECUDA, "cannot allocate the index image (%llu bytes): %s",
+                (unsigned long long)h.total_bytes, cudaGetErrorString(e));
+  }
+  c->blob_bytes = h.total_bytes; c->blob_owned = true; c->hdr = h; c->share_src = nullptr;
+  return MM_OK;
+}
+
+struct blob_guard {
+  mm_ctx *c;
+  ~blob_guard() { if (!c->blob_ready) release_blob(c); }
+};
+
+/* the last writes of an index image: the contig tables (name ids default to -1, groups to 0) and the header; then the
+ * image is ready and the threshold tables go in */
+int finish_blob(mm_ctx *c, const int32_t *contig_len, const int32_t *contig_name_id, const int32_t *contig_group)
+{
+  const mm_blob_header &h = c->hdr;
+  const size_t n = (size_t)h.n_contigs;
+  std::vector<int32_t> tmp(n, -1);
+  CU(c, cudaMemcpyAsync(c->blob + h.off_contig_len, contig_len, n * 4, cudaMemcpyHostToDevice, c->stream));
+  CU(c, cudaMemcpyAsync(c->blob + h.off_contig_name_id, contig_name_id ? contig_name_id : tmp.data(), n * 4, cudaMemcpyHostToDevice, c->stream));
+  CU(c, cudaStreamSynchronize(c->stream)); /* tmp is rewritten below */
+  std::fill(tmp.begin(), tmp.end(), 0);
+  CU(c, cudaMemcpyAsync(c->blob + h.off_contig_group, contig_group ? contig_group : tmp.data(), n * 4, cudaMemcpyHostToDevice, c->stream));
+  CU(c, cudaMemcpyAsync(c->blob, &c->hdr, sizeof(c->hdr), cudaMemcpyHostToDevice, c->stream));
+  CU(c, cudaStreamSynchronize(c->stream));
+  resolve_index(c);
+  c->blob_ready = true;
+  return write_tables(c);
+}
+
 /* wait for the context's stream. Default: cudaStreamSynchronize (spins, lowest latency). With MM_BLOCKING_WAIT=1 the
  * thread sleeps on a blocking event instead -- for hosts with fewer usable CPUs than pipeline threads (DESIGN section 9). */
 cudaError_t wait_stream(mm_ctx *c)
@@ -198,75 +314,31 @@ int prepare_batch_buffers(mm_ctx *c, uint64_t n_bases, uint64_t n_segs)
   int rc;
   /* nibbles: n_bases/2 rounded up to 8-byte groups of 16 bases, + 256 so that the 16-byte-granular bulk copies of the
    * sketch kernel never leave the allocation */
-  const uint64_t pbytes = (n_bases + 15) / 16 * 8;
-  if (pbytes + 256 > c->packed_cap || !c->d_packed) {
-    if (c->d_packed) { cudaFree(c->d_packed); c->d_packed = nullptr; c->packed_cap = 0; }
-    CU(c, cudaMalloc((void **)&c->d_packed, pbytes + 256));
-    c->packed_cap = pbytes + 256;
-    CU(c, cudaMemsetAsync(c->d_packed, 0x88, c->packed_cap, c->stream));
-  }
-  if ((rc = grow(c, c->d_segs, c->segs_cap, n_segs, 1))) return rc;
-  const uint64_t S = (uint64_t)c->params.sketch_size;
-  if (n_segs * S + 1 > c->sk_cap || !c->d_sk_hash) {
-    if (c->d_sk_hash) cudaFree(c->d_sk_hash);
-    if (c->d_sk_val) cudaFree(c->d_sk_val);
-    if (c->d_sk_pos) cudaFree(c->d_sk_pos);
-    if (c->d_sk_strand) cudaFree(c->d_sk_strand);
-    if (c->d_seg_res) cudaFree(c->d_seg_res);
-    if (c->d_sk_reject) cudaFree(c->d_sk_reject);
-    c->d_sk_reject = nullptr;
-    c->d_sk_hash = nullptr; c->d_sk_val = nullptr; c->d_sk_pos = nullptr; c->d_sk_strand = nullptr; c->d_seg_res = nullptr; c->sk_cap = 0;
-    const uint64_t n = n_segs * S + 1;
-    CU(c, cudaMalloc((void **)&c->d_sk_hash, n * 8));
-    CU(c, cudaMalloc((void **)&c->d_sk_val, n * 8));
-    CU(c, cudaMalloc((void **)&c->d_sk_pos, n * 8));
-    CU(c, cudaMalloc((void **)&c->d_sk_strand, n));
-    CU(c, cudaMalloc((void **)&c->d_seg_res, (n_segs + 1) * sizeof(mm_segment_result)));
-    CU(c, cudaMalloc((void **)&c->d_sk_reject, (n_segs + 1) * 4));
-    c->sk_cap = n;
-  }
-  if (!c->d_counters) CU(c, cudaMalloc((void **)&c->d_counters, 64));
+  const uint64_t pbytes = (n_bases + 15) / 16 * 8 + 256;
+  bool fresh = false;
+  if ((rc = c->d_packed.reserve(c, pbytes, pbytes, &fresh))) return rc;
+  if (fresh) CU(c, cudaMemsetAsync(c->d_packed.p, 0x88, c->d_packed.cap, c->stream));
+  const uint64_t n = n_segs * (uint64_t)c->params.sketch_size + 1;
+  if ((rc = c->d_segs.reserve(c, n_segs + 1, n_segs + 1)) || (rc = c->d_sk_hash.reserve(c, n, n)) ||
+      (rc = c->d_sk_val.reserve(c, n, n)) || (rc = c->d_sk_pos.reserve(c, n, n)) || (rc = c->d_sk_strand.reserve(c, n, n)) ||
+      (rc = c->d_seg_res.reserve(c, n_segs + 1, n_segs + 1)) || (rc = c->d_sk_reject.reserve(c, n_segs + 1, n_segs + 1)) ||
+      (rc = c->d_counters.reserve(c, 16, 16)))
+    return rc;
   return MM_OK;
-}
-
-/* experiment (MM_UPLOAD_KERNEL=<CTAs>): the host -> device copy done by a few CTAs that read the pinned host buffer
- * through its unified address (PCIe reads issued by SMs) instead of by the copy engine */
-__global__ void __launch_bounds__(256) k_copy_from_host(uint4 *dst, const uint4 *src, uint64_t n16)
-{
-  const uint64_t stride = (uint64_t)gridDim.x * 256ULL;
-  uint64_t i = (uint64_t)blockIdx.x * 256ULL + threadIdx.x;
-  for (; i + 3 * stride < n16; i += 4 * stride) {
-    const uint4 a = __ldcs(src + i), b = __ldcs(src + i + stride), c = __ldcs(src + i + 2 * stride), d = __ldcs(src + i + 3 * stride);
-    dst[i] = a; dst[i + stride] = b; dst[i + 2 * stride] = c; dst[i + 3 * stride] = d;
-  }
-  for (; i < n16; i += stride) dst[i] = __ldcs(src + i);
 }
 
 /* host -> device copy of `bytes` bytes, in <= 16 MiB pieces when a phase hook is installed (MM_PHASE_UPLOAD_CHUNK) */
 int copy_in(mm_ctx *c, uint8_t *dst, const void *src, uint64_t bytes)
 {
-  static const int skip_after = getenv("MM_SKIP_H2D") ? atoi(getenv("MM_SKIP_H2D")) : 0; /* experiment: timing without the copies */
-  static const int copy_ctas = getenv("MM_UPLOAD_KERNEL") ? atoi(getenv("MM_UPLOAD_KERNEL")) : 0;
-  static std::atomic<int> calls{0};
-  if (skip_after > 0 && calls.fetch_add(1) >= skip_after) return MM_OK;
-  auto one = [&](uint8_t *d, const uint8_t *s_, uint64_t n) -> cudaError_t {
-    if (copy_ctas > 0 && ((uintptr_t)d % 16 == 0) && ((uintptr_t)s_ % 16 == 0)) {
-      const uint64_t n16 = n / 16;
-      if (n16) k_copy_from_host<<<copy_ctas, 256, 0, c->stream>>>((uint4 *)d, (const uint4 *)s_, n16);
-      if (n % 16) return cudaMemcpyAsync(d + n16 * 16, s_ + n16 * 16, n % 16, cudaMemcpyHostToDevice, c->stream);
-      return cudaGetLastError();
-    }
-    return cudaMemcpyAsync(d, s_, n, cudaMemcpyHostToDevice, c->stream);
-  };
   if (!c->hook) {
-    CU(c, one(dst, (const uint8_t *)src, bytes));
+    CU(c, cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, c->stream));
     return MM_OK;
   }
   const uint64_t CH = 16ULL << 20;
   for (uint64_t at = 0; at < bytes; at += CH) {
     const uint64_t n = std::min(CH, bytes - at);
     c->hook(c->hook_user, MM_PHASE_UPLOAD_CHUNK, 1);
-    cudaError_t e = one(dst + at, (const uint8_t *)src + at, n);
+    cudaError_t e = cudaMemcpyAsync(dst + at, (const uint8_t *)src + at, n, cudaMemcpyHostToDevice, c->stream);
     if (e == cudaSuccess) e = wait_stream(c);
     c->hook(c->hook_user, MM_PHASE_UPLOAD_CHUNK, 0);
     CU(c, e);
@@ -281,19 +353,19 @@ int upload_batch(mm_ctx *c, const void *bases, uint64_t n_bases, const mm_segmen
   if (rc) return rc;
   CU(c, cudaSetDevice(c->device));
   if ((rc = prepare_batch_buffers(c, n_bases, n_segs))) return rc;
-  CU(c, cudaEventRecord(c->ev[6], c->stream));
+  CU(c, cudaEventRecord(c->ev[EV_H2D_BEGIN], c->stream));
   if (packed) {
     const uint64_t pbytes = (n_bases + 1) / 2;
-    if ((rc = copy_in(c, c->d_packed, bases, pbytes))) return rc;
-    CU(c, cudaMemsetAsync(c->d_packed + pbytes, 0x88, 64, c->stream));
+    if ((rc = copy_in(c, c->d_packed.p, bases, pbytes))) return rc;
+    CU(c, cudaMemsetAsync(c->d_packed.p + pbytes, 0x88, 64, c->stream));
     if (n_bases & 1) { /* the unused high nibble of the last byte is whatever the caller had there: irrelevant (never a k-mer) */ }
   } else {
-    if ((rc = grow(c, c->d_bases, c->bases_cap, n_bases, 256))) return rc;
-    if ((rc = copy_in(c, c->d_bases, bases, n_bases))) return rc;
-    CU(c, cudaMemsetAsync(c->d_bases + n_bases, 'N', 256, c->stream));
+    if ((rc = c->d_bases.reserve(c, n_bases + 256, n_bases + 256))) return rc;
+    if ((rc = copy_in(c, c->d_bases.p, bases, n_bases))) return rc;
+    CU(c, cudaMemsetAsync(c->d_bases.p + n_bases, 'N', 256, c->stream));
   }
-  CU(c, cudaMemcpyAsync(c->d_segs, segs, n_segs * sizeof(mm_segment), cudaMemcpyHostToDevice, c->stream));
-  CU(c, cudaEventRecord(c->ev[7], c->stream));
+  CU(c, cudaMemcpyAsync(c->d_segs.p, segs, n_segs * sizeof(mm_segment), cudaMemcpyHostToDevice, c->stream));
+  CU(c, cudaEventRecord(c->ev[EV_H2D_END], c->stream));
   c->n_bases = n_bases;
   c->n_segs = n_segs;
   c->batch_is_ascii = !packed;
@@ -305,7 +377,7 @@ int upload_batch(mm_ctx *c, const void *bases, uint64_t n_bases, const mm_segmen
 int launch_pack_if_ascii(mm_ctx *c)
 {
   if (!c->batch_is_ascii) { c->pack_ms = 0; return MM_OK; }
-  CU(c, mm_launch_pack_bases(c->d_bases, c->d_packed, c->n_bases, c->stream, c->sm_count));
+  CU(c, mm_launch_pack_bases(c->d_bases.p, c->d_packed.p, c->n_bases, c->stream, c->sm_count));
   c->launches++;
   return MM_OK;
 }
@@ -313,16 +385,16 @@ int launch_pack_if_ascii(mm_ctx *c)
 mm_dev_batch make_batch(mm_ctx *c)
 {
   mm_dev_batch b{};
-  b.bases = c->d_bases; b.packed = c->d_packed; b.segs = c->d_segs; b.n_segs = (uint32_t)c->n_segs;
-  b.sk_hash = c->d_sk_hash; b.sk_val = c->d_sk_val; b.sk_pos = c->d_sk_pos; b.sk_strand = c->d_sk_strand;
-  b.seg_res = c->d_seg_res; b.sk_reject = c->d_sk_reject;
-  b.cands = c->d_cands; b.cand_cap = (uint32_t)std::min<uint64_t>(c->cand_cap, 0xffffffffu);
-  b.loci = c->d_loci; b.loci_cap = (uint32_t)std::min<uint64_t>(c->loci_cap, 0xffffffffu);
-  b.counters = c->d_counters;
-  b.scratch = c->d_scratch; b.scratch_slice = c->scratch_slice; b.scratch_pool_off = c->scratch_pool;
-  b.scratch_cap = c->scratch_cap;
-  b.l2_ranges = c->d_l2_ranges; b.l2_rec_off = c->d_l2_rec_off; b.l2_recs = c->d_l2_recs; b.l2_recs_cap = c->l2_recs_cap;
-  b.l2_loci_per_cand = 2;
+  b.bases = c->d_bases.p; b.packed = c->d_packed.p; b.segs = c->d_segs.p; b.n_segs = (uint32_t)c->n_segs;
+  b.sk_hash = c->d_sk_hash.p; b.sk_val = c->d_sk_val.p; b.sk_pos = c->d_sk_pos.p; b.sk_strand = c->d_sk_strand.p;
+  b.seg_res = c->d_seg_res.p; b.sk_reject = c->d_sk_reject.p;
+  b.cands = c->d_cands.p; b.cand_cap = (uint32_t)std::min<uint64_t>(c->d_cands.cap, 0xffffffffu);
+  b.loci = c->d_loci.p; b.loci_cap = (uint32_t)std::min<uint64_t>(c->d_loci.cap, 0xffffffffu);
+  b.counters = c->d_counters.p;
+  b.scratch = c->d_scratch.p; b.scratch_slice = c->scratch_slice; b.scratch_pool_off = c->scratch_pool;
+  b.scratch_cap = c->d_scratch.cap;
+  b.l2_ranges = c->d_l2_ranges.p; b.l2_rec_off = c->d_l2_rec_off.p; b.l2_recs = c->d_l2_recs.p; b.l2_recs_cap = c->d_l2_recs.cap;
+  b.l2_loci_per_cand = L2_LOCI_PER_CAND;
   return b;
 }
 
@@ -334,10 +406,7 @@ int ensure_scratch(mm_ctx *c, uint64_t pool_elems)
   }
   const uint64_t slice = 3ULL << 16; /* 65536 points per CTA slice */
   const uint64_t need = slice * c->l1_grid + pool_elems;
-  if (c->d_scratch && c->scratch_cap >= need) return MM_OK;
-  if (c->d_scratch) { cudaFree(c->d_scratch); c->d_scratch = nullptr; }
-  CU(c, cudaMalloc((void **)&c->d_scratch, need * 8));
-  c->scratch_cap = need;
+  if (int rc = c->d_scratch.reserve(c, need, need)) return rc;
   c->scratch_slice = slice;
   c->scratch_pool = slice * c->l1_grid;
   return MM_OK;
@@ -366,62 +435,75 @@ int read_words(mm_ctx *c, const void *dev, uint32_t *out, int n_words)
 }
 #define RD(c, dev, out, n) do { int rc__ = read_words((c), (dev), (out), (n)); if (rc__) return rc__; } while (0)
 
+/* K3's general kernel (mm_l2.cu), over every candidate or (only_flagged) over the ones the stream kernels flagged, whose
+ * loci it appends after the fixed slots. The counters come back in h_cnt. *grown: the locus buffer was too small and has
+ * been grown; the caller runs the kernel again. */
+int run_l2_general(mm_ctx *c, bool only_flagged, uint32_t *h_cnt, bool *grown)
+{
+  const mm_dev_batch b = make_batch(c);
+  const uint32_t nc = (uint32_t)c->n_cands;
+  *grown = false;
+  if (only_flagged) { /* counter 1 was zeroed in front of the stream kernels */
+    k_set_u32<<<1, 1, 0, c->stream>>>(c->d_counters.p + 6, nc * L2_LOCI_PER_CAND);
+    c->launches++;
+    CU(c, mm_launch_l2_overflow(c->params, c->ix, b, nc, c->stream, c->sm_count));
+    c->launches++;
+  } else {
+    ZERO_WORDS(c, c->d_counters.p + 1, 1);
+    ZERO_WORDS(c, c->d_counters.p + 6, 2);
+    CU(c, cudaEventRecord(c->ev[EV_K3_BEGIN], c->stream));
+    CU(c, mm_launch_l2(c->params, c->ix, b, nc, c->stream, c->sm_count));
+    CU(c, cudaEventRecord(c->ev[EV_K3_END], c->stream));
+    if (nc) c->launches++;
+  }
+  RD(c, c->d_counters.p, h_cnt, 16);
+  if (h_cnt[1] == 2) return fail(c, MM_ECUDA, "L2 live-set overflow in the general kernel: the reference index has more than "
+                                 "sketch_size+64 overlapping minmer windows at one position");
+  if (h_cnt[1] == 1 || h_cnt[6] > c->d_loci.cap) {
+    if (int rc = c->d_loci.reserve(c, h_cnt[6], (uint64_t)h_cnt[6] + h_cnt[6] / 4 + 1024)) return rc;
+    *grown = true;
+  }
+  return MM_OK;
+}
+
 /* K3 fast path (mm_l2_stream.cu): ranges+scan -> records -> lane-per-candidate scan -> general kernel for the
  * candidates that need more locus slots. Returns MM_ENOMEM if the record buffer cannot be allocated. */
 int run_l2_stream(mm_ctx *c, uint32_t *h_cnt)
 {
   const uint64_t nc = c->n_cands;
-  const uint32_t LPC = 2;
-  CU(c, cudaEventRecord(c->ev[3], c->stream));
+  int rc;
+  CU(c, cudaEventRecord(c->ev[EV_K3_BEGIN], c->stream));
   if (nc == 0) {
-    CU(c, cudaEventRecord(c->ev[4], c->stream));
+    CU(c, cudaEventRecord(c->ev[EV_K3_END], c->stream));
     CU(c, wait_stream(c));
     c->n_loci = 0;
     return MM_OK;
   }
   if (nc + 1 > c->l2_cand_cap) {
-    if (c->d_l2_ranges) cudaFree(c->d_l2_ranges);
-    if (c->d_l2_rec_off) cudaFree(c->d_l2_rec_off);
-    if (c->d_scan_tmp) cudaFree(c->d_scan_tmp);
-    c->d_l2_ranges = nullptr; c->d_l2_rec_off = nullptr; c->d_scan_tmp = nullptr;
-    c->l2_cand_cap = nc + nc / 8 + 1024;
-    CU(c, cudaMalloc((void **)&c->d_l2_ranges, c->l2_cand_cap * sizeof(mm_l2_range)));
-    CU(c, cudaMalloc((void **)&c->d_l2_rec_off, (c->l2_cand_cap + 1) * 8));
-    c->scan_tmp_bytes = mm_l2_scan_tmp_bytes((uint32_t)c->l2_cand_cap);
-    CU(c, cudaMalloc(&c->d_scan_tmp, c->scan_tmp_bytes + 256));
-    if (c->d_l2_order) cudaFree(c->d_l2_order);
-    c->d_l2_order = nullptr;
-    c->l2_order_bytes = mm_l2_order_bytes((uint32_t)c->l2_cand_cap);
-    CU(c, cudaMalloc(&c->d_l2_order, c->l2_order_bytes));
+    const uint64_t cap = nc + nc / 8 + 1024;
+    const uint64_t scan_bytes = mm_l2_scan_tmp_bytes((uint32_t)cap) + 256, order_bytes = mm_l2_order_bytes((uint32_t)cap);
+    if ((rc = c->d_l2_ranges.reserve(c, cap, cap)) || (rc = c->d_l2_rec_off.reserve(c, cap + 1, cap + 1)) ||
+        (rc = c->d_scan_tmp.reserve(c, scan_bytes, scan_bytes)) || (rc = c->d_l2_order.reserve(c, order_bytes, order_bytes)))
+      return rc;
+    c->l2_cand_cap = cap;
   }
-  if (c->loci_cap < nc * LPC + 1024) {
-    if (c->d_loci) cudaFree(c->d_loci);
-    c->d_loci = nullptr;
-    c->loci_cap = nc * LPC + nc / 8 + 4096;
-    CU(c, cudaMalloc((void **)&c->d_loci, c->loci_cap * sizeof(mm_l2_locus)));
-  }
+  if ((rc = c->d_loci.reserve(c, nc * L2_LOCI_PER_CAND + 1024, nc * L2_LOCI_PER_CAND + nc / 8 + 4096))) return rc;
   mm_dev_batch b = make_batch(c);
   const auto tk0 = std::chrono::steady_clock::now();
-  ZERO_WORDS(c, c->d_l2_rec_off + nc, 2);
-  CU(c, mm_launch_l2_ranges(c->params, c->ix, b, (uint32_t)nc, c->d_scan_tmp, c->scan_tmp_bytes + 256, c->stream));
+  ZERO_WORDS(c, c->d_l2_rec_off.p + nc, 2);
+  CU(c, mm_launch_l2_ranges(c->params, c->ix, b, (uint32_t)nc, c->d_scan_tmp.p, c->d_scan_tmp.cap, c->stream));
   uint64_t total = 0;
-  RD(c, c->d_l2_rec_off + nc, (uint32_t *)&total, 2);
+  RD(c, c->d_l2_rec_off.p + nc, (uint32_t *)&total, 2);
   const auto tk1 = std::chrono::steady_clock::now();
   c->stage_ms[6] = std::chrono::duration<float, std::milli>(tk1 - tk0).count(); /* host view: ranges + scan + readback */
-  if (total + 64 > c->l2_recs_cap) { /* the scan's record readers run up to 2 * RING_CHUNKS + 2 records past a stream's end */
-    if (c->d_l2_recs) cudaFree(c->d_l2_recs);
-    c->d_l2_recs = nullptr; c->l2_recs_cap = 0;
-    const uint64_t want = total + total / 16 + 1024;
-    if (cudaMalloc((void **)&c->d_l2_recs, want * sizeof(uint2)) != cudaSuccess) {
-      cudaGetLastError();
-      return fail(c, MM_ENOMEM, "cannot allocate %llu L2 operation records", (unsigned long long)want);
-    }
-    c->l2_recs_cap = want;
-  }
+  /* the scan's record readers run up to 2 * RING_CHUNKS + 2 records past a stream's end */
+  const uint64_t want = total + total / 16 + 1024;
+  if (c->d_l2_recs.reserve(c, total + 64, want))
+    return fail(c, MM_ENOMEM, "cannot allocate %llu L2 operation records", (unsigned long long)want);
   for (int attempt = 0; attempt < 4; attempt++) {
     b = make_batch(c);
-    ZERO_WORDS(c, c->d_counters + 1, 1);
-    ZERO_WORDS(c, c->d_counters + 6, 2);
+    ZERO_WORDS(c, c->d_counters.p + 1, 1);
+    ZERO_WORDS(c, c->d_counters.p + 6, 2);
     /* the record-preparation kernel is the bandwidth-bound one: no PCIe upload next to it (MM_PHASE_L2) */
     {
       struct phase_guard { /* the hook is always closed, whatever fails in between */
@@ -430,46 +512,69 @@ int run_l2_stream(mm_ctx *c, uint32_t *h_cnt)
         void close() { if (open) { c->hook(c->hook_user, MM_PHASE_L2, 0); open = false; } }
         ~phase_guard() { close(); }
       } guard(c);
-      CU(c, cudaEventRecord(c->ev[8], c->stream));
+      CU(c, cudaEventRecord(c->ev[EV_PREP_BEGIN], c->stream));
       CU(c, mm_launch_l2_prep(c->params, c->ix, b, (uint32_t)nc, c->stream, c->sm_count));
-      CU(c, cudaEventRecord(c->ev[9], c->stream));
+      CU(c, cudaEventRecord(c->ev[EV_PREP_END], c->stream));
       if (guard.open && c->blocking_wait) CU(c, cudaEventRecord(c->ev_wait, c->stream));
       uint32_t *perm = nullptr;
-      CU(c, mm_launch_l2_order(b, (uint32_t)nc, c->d_l2_order, c->l2_order_bytes, &perm, c->stream));
+      CU(c, mm_launch_l2_order(b, (uint32_t)nc, c->d_l2_order.p, c->d_l2_order.cap, &perm, c->stream));
       b.l2_perm = perm;
       CU(c, mm_launch_l2_scan(c->params, c->ix, b, (uint32_t)nc, c->stream, c->sm_count));
       /* the scan is already queued behind it: waiting for the end of the preparation kernel costs no bubble */
-      if (guard.open) CU(c, cudaEventSynchronize(c->blocking_wait ? c->ev_wait : c->ev[9]));
+      if (guard.open) CU(c, cudaEventSynchronize(c->blocking_wait ? c->ev_wait : c->ev[EV_PREP_END]));
     }
     c->launches += 4; /* own kernels: ranges, prep, order keys, scan (the prefix sum and the sort are library calls, not counted) */
-    RD(c, c->d_counters, h_cnt, 16);
-    uint64_t extent = nc * LPC;
-    if (h_cnt[7] > 0) { /* candidates with more than LPC loci: general kernel, loci appended after the fixed slots */
+    RD(c, c->d_counters.p, h_cnt, 16);
+    uint64_t extent = nc * L2_LOCI_PER_CAND;
+    if (h_cnt[7] > 0) { /* candidates with more than L2_LOCI_PER_CAND loci: general kernel, loci appended after the fixed slots */
       c->diag[MM_DIAG_L2_GENERAL_CANDS] += h_cnt[7];
-      const uint32_t base = (uint32_t)extent;
-      k_set_u32<<<1, 1, 0, c->stream>>>(c->d_counters + 6, base);
-      c->launches++;
-      CU(c, mm_launch_l2_overflow(c->params, c->ix, b, (uint32_t)nc, c->stream, c->sm_count));
-      c->launches += 1;
-      RD(c, c->d_counters, h_cnt, 16);
-      if (h_cnt[1] == 2) return fail(c, MM_ECUDA, "L2 live-set overflow in the general kernel");
-      if (h_cnt[1] == 1 || h_cnt[6] > c->loci_cap) { /* grow and redo prep+scan+overflow */
+      bool grown = false;
+      if ((rc = run_l2_general(c, true, h_cnt, &grown))) return rc;
+      if (grown) { /* redo prep+scan+overflow */
         c->diag[MM_DIAG_L2_LOCI_REGROW]++;
-        cudaFree(c->d_loci); c->d_loci = nullptr;
-        c->loci_cap = (uint64_t)h_cnt[6] + h_cnt[6] / 4 + 1024;
-        CU(c, cudaMalloc((void **)&c->d_loci, c->loci_cap * sizeof(mm_l2_locus)));
         continue;
       }
       extent = h_cnt[6];
     }
-    CU(c, cudaEventRecord(c->ev[4], c->stream));
+    CU(c, cudaEventRecord(c->ev[EV_K3_END], c->stream));
     CU(c, wait_stream(c));
-    cudaEventElapsedTime(&c->stage_ms[6], c->ev[8], c->ev[9]); /* k_l2_prep */
-    cudaEventElapsedTime(&c->stage_ms[7], c->ev[9], c->ev[4]); /* k_l2_scan (+ overflow kernel) */
+    cudaEventElapsedTime(&c->stage_ms[6], c->ev[EV_PREP_BEGIN], c->ev[EV_PREP_END]); /* k_l2_prep */
+    cudaEventElapsedTime(&c->stage_ms[7], c->ev[EV_PREP_END], c->ev[EV_K3_END]);     /* k_l2_scan (+ overflow kernel) */
     c->n_loci = extent;
     return MM_OK;
   }
   return fail(c, MM_ECUDA, "locus buffer kept overflowing");
+}
+
+/* K3: the stream kernels, or the general kernel alone (MM_L2_GENERAL, large sketches, or no memory for the stream
+ * kernels' records), retried alone while the locus buffer is too small (it is idempotent) */
+int run_l2(mm_ctx *c)
+{
+  uint32_t h_cnt[16];
+  if (c->l2_mode == 1) {
+    const int rc = run_l2_stream(c, h_cnt);
+    if (rc != MM_ENOMEM) return rc;
+    /* not enough memory for the operation records: fall through to the general kernel */
+  }
+  for (int attempt = 0; attempt < 4; attempt++) {
+    bool grown = false;
+    if (int rc = run_l2_general(c, false, h_cnt, &grown)) return rc;
+    if (!grown) {
+      c->n_loci = h_cnt[6];
+      return MM_OK;
+    }
+  }
+  return fail(c, MM_ECUDA, "locus buffer kept overflowing");
+}
+
+/* stage_ms / pack_ms of the batch run_pipeline has just mapped */
+void record_stage_times(mm_ctx *c)
+{
+  if (c->batch_is_ascii) cudaEventElapsedTime(&c->pack_ms, c->ev[EV_BEGIN], c->ev[EV_K1_BEGIN]);
+  cudaEventElapsedTime(&c->stage_ms[0], c->ev[EV_K1_BEGIN], c->ev[EV_K1_END]);
+  cudaEventElapsedTime(&c->stage_ms[1], c->ev[EV_K1_END], c->ev[EV_K2_END]);
+  cudaEventElapsedTime(&c->stage_ms[2], c->ev[EV_K3_BEGIN], c->ev[EV_K3_END]);
+  cudaEventElapsedTime(&c->stage_ms[5], c->ev[EV_BEGIN], c->ev[EV_K3_END]); /* first launch -> last kernel end, incl. host gaps */
 }
 
 /* K1 -> K2 -> K3 on the resident batch, growing output buffers and retrying on overflow */
@@ -479,103 +584,46 @@ int run_pipeline(mm_ctx *c)
   if (rc) return rc;
   CU(c, cudaSetDevice(c->device));
   const uint64_t n_segs = c->n_segs;
-  if (c->cand_cap < 2 * n_segs + 1024) {
-    if (c->d_cands) { cudaFree(c->d_cands); c->d_cands = nullptr; }
-    c->cand_cap = 2 * n_segs + 1024;
-    CU(c, cudaMalloc((void **)&c->d_cands, c->cand_cap * sizeof(mm_l1_candidate)));
-  }
-  if (c->loci_cap < 2 * c->cand_cap) {
-    if (c->d_loci) { cudaFree(c->d_loci); c->d_loci = nullptr; }
-    c->loci_cap = 2 * c->cand_cap;
-    CU(c, cudaMalloc((void **)&c->d_loci, c->loci_cap * sizeof(mm_l2_locus)));
-  }
-  uint64_t pool0 = 32ULL << 20; /* interval points the bump pool holds at first (grown on demand below) */
-  if (const char *e = getenv("MM_L1_POOL_ELEMS")) pool0 = std::max<uint64_t>(1024, strtoull(e, nullptr, 10)); /* tests: force the regrow path */
-  if ((rc = ensure_scratch(c, c->scratch_cap ? c->scratch_cap - c->scratch_pool : pool0))) return rc;
-  if (c->l1_slow_cap < n_segs + 1) {
-    if (c->d_l1_slow) cudaFree(c->d_l1_slow);
-    c->d_l1_slow = nullptr;
-    c->l1_slow_cap = n_segs + n_segs / 8 + 1024;
-    CU(c, cudaMalloc((void **)&c->d_l1_slow, c->l1_slow_cap * 4));
-  }
+  if ((rc = c->d_cands.reserve(c, 2 * n_segs + 1024, 2 * n_segs + 1024)) ||
+      (rc = c->d_loci.reserve(c, 2 * c->d_cands.cap, 2 * c->d_cands.cap)) ||
+      (rc = ensure_scratch(c, c->d_scratch.cap ? c->d_scratch.cap - c->scratch_pool : c->l1_pool0)) ||
+      (rc = c->d_l1_slow.reserve(c, n_segs + 1, n_segs + n_segs / 8 + 1024)))
+    return rc;
 
   uint32_t h_cnt[16];
   for (int attempt = 0; attempt < 6; attempt++) {
     mm_dev_batch b = make_batch(c);
-    ZERO_WORDS(c, c->d_counters, 16);
-    CU(c, cudaEventRecord(c->ev[0], c->stream));
+    ZERO_WORDS(c, c->d_counters.p, 16);
+    CU(c, cudaEventRecord(c->ev[EV_BEGIN], c->stream));
     if ((rc = launch_pack_if_ascii(c))) return rc;
-    CU(c, cudaEventRecord(c->ev_pack, c->stream));
+    CU(c, cudaEventRecord(c->ev[EV_K1_BEGIN], c->stream));
     CU(c, mm_launch_sketch(c->params, b, c->stream, c->sm_count, c->sk_mode));
-    CU(c, cudaEventRecord(c->ev[1], c->stream));
+    CU(c, cudaEventRecord(c->ev[EV_K1_END], c->stream));
     int l1_launches = 0;
-    CU(c, mm_launch_l1(c->params, c->ix, b, c->stream, c->sm_count, c->d_l1_slow, c->l1_warp, &l1_launches));
-    CU(c, cudaEventRecord(c->ev[2], c->stream));
+    CU(c, mm_launch_l1(c->params, c->ix, b, c->stream, c->sm_count, c->d_l1_slow.p, c->l1_warp, &l1_launches));
+    CU(c, cudaEventRecord(c->ev[EV_K2_END], c->stream));
     c->launches += (c->sk_mode ? 1 : 2) + (uint64_t)l1_launches;
-    RD(c, c->d_counters, h_cnt, 16);
+    RD(c, c->d_counters.p, h_cnt, 16);
     const uint64_t need_cands = h_cnt[0];
     bool retry = false;
     c->diag[MM_DIAG_L1_CTA_SEGMENTS] += h_cnt[8];
     c->diag[MM_DIAG_SKETCH_GENERAL_SEGMENTS] += h_cnt[9];
-    if (h_cnt[3] || need_cands > c->cand_cap) {
+    if (h_cnt[3] || need_cands > c->d_cands.cap) {
       c->diag[MM_DIAG_CAND_REGROW]++;
-      cudaFree(c->d_cands); c->d_cands = nullptr;
-      c->cand_cap = need_cands + need_cands / 4 + 1024;
-      CU(c, cudaMalloc((void **)&c->d_cands, c->cand_cap * sizeof(mm_l1_candidate)));
+      if ((rc = c->d_cands.reserve(c, need_cands, need_cands + need_cands / 4 + 1024))) return rc;
       retry = true;
     }
     if (h_cnt[2]) { /* scratch pool exhausted: quadruple it */
       c->diag[MM_DIAG_L1_POOL_REGROW]++;
-      const uint64_t pool = c->scratch_cap - c->scratch_pool;
-      cudaFree(c->d_scratch); c->d_scratch = nullptr; c->scratch_cap = 0;
-      if ((rc = ensure_scratch(c, pool * 4))) return rc;
+      if ((rc = ensure_scratch(c, (c->d_scratch.cap - c->scratch_pool) * 4))) return rc;
       retry = true;
     }
     if (retry) continue;
     c->n_cands = need_cands;
-    /* K3 */
-    if (c->l2_mode == 1) {
-      int rc2 = run_l2_stream(c, h_cnt);
-      if (rc2 == MM_OK) {
-        if (c->batch_is_ascii) cudaEventElapsedTime(&c->pack_ms, c->ev[0], c->ev_pack);
-        cudaEventElapsedTime(&c->stage_ms[0], c->ev_pack, c->ev[1]);
-        cudaEventElapsedTime(&c->stage_ms[1], c->ev[1], c->ev[2]);
-        cudaEventElapsedTime(&c->stage_ms[2], c->ev[3], c->ev[4]);
-        cudaEventElapsedTime(&c->stage_ms[5], c->ev[0], c->ev[4]);
-        c->batch_mapped = true;
-        return MM_OK;
-      }
-      if (rc2 != MM_ENOMEM) return rc2;
-      /* not enough memory for the operation records: fall through to the general kernel */
-    }
-    /* general kernel, retried alone if the locus buffer is too small (it is idempotent) */
-    for (int a2 = 0; a2 < 4; a2++) {
-      b = make_batch(c);
-      ZERO_WORDS(c, c->d_counters + 1, 1);
-      ZERO_WORDS(c, c->d_counters + 6, 2);
-      CU(c, cudaEventRecord(c->ev[3], c->stream));
-      CU(c, mm_launch_l2(c->params, c->ix, b, (uint32_t)c->n_cands, c->stream, c->sm_count));
-      CU(c, cudaEventRecord(c->ev[4], c->stream));
-      if (c->n_cands) c->launches += 1;
-      RD(c, c->d_counters, h_cnt, 16);
-      if (h_cnt[1] == 2) return fail(c, MM_ECUDA, "L2 live-set overflow: the reference index has more than "
-                                     "sketch_size+64 overlapping minmer windows at one position");
-      if (h_cnt[1] == 1 || h_cnt[6] > c->loci_cap) {
-        cudaFree(c->d_loci); c->d_loci = nullptr;
-        c->loci_cap = (uint64_t)h_cnt[6] + h_cnt[6] / 4 + 1024;
-        CU(c, cudaMalloc((void **)&c->d_loci, c->loci_cap * sizeof(mm_l2_locus)));
-        continue;
-      }
-      c->n_loci = h_cnt[6];
-      if (c->batch_is_ascii) cudaEventElapsedTime(&c->pack_ms, c->ev[0], c->ev_pack);
-      cudaEventElapsedTime(&c->stage_ms[0], c->ev_pack, c->ev[1]);
-      cudaEventElapsedTime(&c->stage_ms[1], c->ev[1], c->ev[2]);
-      cudaEventElapsedTime(&c->stage_ms[2], c->ev[3], c->ev[4]);
-      cudaEventElapsedTime(&c->stage_ms[5], c->ev[0], c->ev[4]); /* first launch -> last kernel end, incl. host gaps */
-      c->batch_mapped = true;
-      return MM_OK;
-    }
-    return fail(c, MM_ECUDA, "locus buffer kept overflowing");
+    if ((rc = run_l2(c))) return rc;
+    record_stage_times(c);
+    c->batch_mapped = true;
+    return MM_OK;
   }
   return fail(c, MM_ECUDA, "candidate/scratch buffers kept overflowing");
 }
@@ -618,8 +666,7 @@ int mm_ctx_create(int device, const mm_params *params, mm_ctx **out)
     delete c;
     return fail(nullptr, MM_ECUDA, "cannot create stream");
   }
-  for (auto &ev : c->ev) cudaEventCreate(&ev);
-  cudaEventCreate(&c->ev_pack);
+  for (cudaEvent_t &ev : c->ev.ev) cudaEventCreate(&ev);
   if (cudaHostAlloc((void **)&c->h_pub, 256, cudaHostAllocMapped | cudaHostAllocPortable) != cudaSuccess) {
     cudaStreamDestroy(c->stream);
     delete c;
@@ -632,6 +679,7 @@ int mm_ctx_create(int device, const mm_params *params, mm_ctx **out)
   if (const char *g = getenv("MM_L2_GENERAL")) c->l2_mode = (g[0] == '1') ? 0 : 1; /* test hook: general kernel only */
   if (const char *g = getenv("MM_SKETCH_TABLE")) c->sk_mode = (g[0] == '1') ? 1 : 0; /* test hook: general sketch kernel only */
   if (const char *g = getenv("MM_L1_CTA")) c->l1_warp = (g[0] == '1') ? 0 : 1; /* test hook: general L1 path only */
+  if (const char *g = getenv("MM_L1_POOL_ELEMS")) c->l1_pool0 = std::max<uint64_t>(1024, strtoull(g, nullptr, 10)); /* test hook: force the pool regrow */
   if (params->sketch_size > 1000) c->l2_mode = 0; /* the stream kernel packs its counters in 11 bits */
   *out = c;
   return MM_OK;
@@ -642,16 +690,12 @@ int mm_ctx_destroy(mm_ctx *c)
   if (!c) return MM_OK;
   cudaSetDevice(c->device);
   cudaStreamSynchronize(c->stream);
-  if (c->blob && c->blob_owned) cudaFree(c->blob);
+  release_blob(c);
   mm_built_index_free(&c->built);
-  cudaFree(c->d_bases); cudaFree(c->d_packed); cudaFree(c->d_sk_reject); cudaFree(c->d_segs); cudaFree(c->d_sk_hash); cudaFree(c->d_sk_val); cudaFree(c->d_sk_pos); cudaFree(c->d_sk_strand);
-  cudaFree(c->d_seg_res); cudaFree(c->d_cands); cudaFree(c->d_loci); cudaFree(c->d_counters); cudaFree(c->d_scratch);
-  cudaFree(c->d_l1_slow); cudaFree(c->d_l2_order); cudaFree(c->d_l2_ranges); cudaFree(c->d_l2_rec_off); cudaFree(c->d_l2_recs); cudaFree(c->d_scan_tmp);
-  for (auto &ev : c->ev) cudaEventDestroy(ev);
   if (c->h_pub) cudaFreeHost(c->h_pub);
   if (c->ev_wait) cudaEventDestroy(c->ev_wait);
   cudaStreamDestroy(c->stream);
-  delete c;
+  delete c; /* the batch buffers and the timing events go with it */
   return MM_OK;
 }
 
@@ -675,18 +719,7 @@ int mm_index_upload(mm_ctx *c, const mm_minmer *mi, uint64_t n_mi, const uint64_
   if (n_keys && (!keys || !offsets || !key_is_freq)) return fail(c, MM_EINVAL, "null lookup arrays");
   if (n_keys && offsets[n_keys] != n_points) return fail(c, MM_EINVAL, "offsets[n_keys] != n_points");
   CU(c, cudaSetDevice(c->device));
-  if (c->blob && c->blob_owned) { cudaFree(c->blob); }
-  c->blob = nullptr; c->blob_ready = false;
-  /* every early return below releases the temporaries (dev_tmp) and the half-built image (blob_guard) */
-  struct dev_tmp {
-    void *p = nullptr;
-    ~dev_tmp() { if (p) cudaFree(p); }
-  };
-  struct blob_guard {
-    mm_ctx *c;
-    bool done = false;
-    ~blob_guard() { if (!done && c->blob && c->blob_owned) { cudaFree(c->blob); c->blob = nullptr; c->blob_bytes = 0; c->blob_ready = false; } }
-  } guard{c};
+  release_blob(c);
 
   /* contig_start: first index entry of each contig; the index must be ordered by (seqId, wpos) */
   std::vector<uint64_t> cstart((size_t)n_contigs + 1, 0);
@@ -703,44 +736,21 @@ int mm_index_upload(mm_ctx *c, const mm_minmer *mi, uint64_t n_mi, const uint64_
     }
     for (int32_t s = 0; s < n_contigs; s++) cstart[(size_t)s + 1] += cstart[(size_t)s];
   }
-  int tab_log2 = 4;
-  while ((1ULL << tab_log2) < 2 * n_keys + 2) tab_log2++;
-  const uint64_t tab_slots = 1ULL << tab_log2;
-
-  mm_blob_header h{};
-  h.magic = MM_BLOB_MAGIC;
-  h.n_minmers = n_mi; h.n_keys = n_keys; h.n_points = n_points;
-  h.n_contigs = n_contigs; h.tab_log2 = tab_log2;
-  uint64_t o = align_up(sizeof(mm_blob_header), 256);
-  auto place = [&](uint64_t bytes) { uint64_t at = o; o = align_up(o + bytes, 256); return at; };
-  h.off_idx_hash = place((n_mi + 1) * 8);
-  h.off_idx_wpos = place((n_mi + 1) * 4);
-  h.off_idx_wend = place((n_mi + 1) * 4);
-  h.off_idx_strand = place(n_mi + 1);
-  h.off_contig_start = place(((uint64_t)n_contigs + 1) * 8);
-  h.off_idx2_hash = place((n_mi + 1) * 8);
-  h.off_idx2_wend = place((n_mi + 1) * 4);
-  h.off_tab = place(tab_slots * sizeof(mm_tab_slot));
-  h.off_pts = place((n_points + 1) * 8);
-  h.off_contig_len = place((uint64_t)n_contigs * 4);
-  h.off_contig_name_id = place((uint64_t)n_contigs * 4);
-  h.off_contig_group = place((uint64_t)n_contigs * 4);
-  h.off_cutoffs = place(TABLE_REGION_BYTES);
-  h.off_min_hits = place(TABLE_REGION_BYTES);
-  h.total_bytes = o;
-  CU(c, cudaMalloc((void **)&c->blob, o));
-  c->blob_bytes = o; c->blob_owned = true; c->hdr = h; c->share_src = nullptr;
+  const mm_blob_header h = blob_layout(n_mi, n_keys, n_points, n_contigs);
+  const uint64_t tab_slots = 1ULL << h.tab_log2;
+  int rc = replace_blob(c, h);
+  if (rc) return rc;
+  blob_guard guard{c}; /* every early return below also releases the temporaries (dev_array) */
 
   /* AoS records go up in chunks and are re-laid out on the device (SoA index, packed points, hash table) */
   {
     const uint64_t CH = 1ULL << 24;
-    dev_tmp stage_buf;
-    CU(c, cudaMalloc(&stage_buf.p, CH * 24));
-    void *stage = stage_buf.p;
+    dev_array<uint8_t> stage;
+    if ((rc = stage.reserve(c, CH * 24, CH * 24))) return rc;
     for (uint64_t at = 0; at < n_mi; at += CH) {
       const uint64_t n = std::min(CH, n_mi - at);
-      CU(c, cudaMemcpyAsync(stage, mi + at, n * sizeof(mm_minmer), cudaMemcpyHostToDevice, c->stream));
-      CU(c, mm_upload_split_minmers((const mm_minmer *)stage, n, (uint64_t *)(c->blob + h.off_idx_hash) + at,
+      CU(c, cudaMemcpyAsync(stage.p, mi + at, n * sizeof(mm_minmer), cudaMemcpyHostToDevice, c->stream));
+      CU(c, mm_upload_split_minmers((const mm_minmer *)stage.p, n, (uint64_t *)(c->blob + h.off_idx_hash) + at,
                                     (int32_t *)(c->blob + h.off_idx_wpos) + at, (int32_t *)(c->blob + h.off_idx_wend) + at,
                                     (int8_t *)(c->blob + h.off_idx_strand) + at, c->stream));
       CU(c, cudaStreamSynchronize(c->stream));
@@ -750,51 +760,38 @@ int mm_index_upload(mm_ctx *c, const mm_minmer *mi, uint64_t n_mi, const uint64_
     CU(c, mm_build_death_order((const uint64_t *)(c->blob + h.off_idx_hash), (const int32_t *)(c->blob + h.off_idx_wend),
                                (const uint64_t *)(c->blob + h.off_contig_start), n_contigs, n_mi,
                                (uint64_t *)(c->blob + h.off_idx2_hash), (int32_t *)(c->blob + h.off_idx2_wend), c->stream));
-    dev_tmp err_buf;
-    CU(c, cudaMalloc(&err_buf.p, 4));
-    uint32_t *d_err = (uint32_t *)err_buf.p;
-    CU(c, cudaMemsetAsync(d_err, 0, 4, c->stream));
+    dev_array<uint32_t> d_err;
+    if ((rc = d_err.reserve(c, 1, 1))) return rc;
+    CU(c, cudaMemsetAsync(d_err.p, 0, 4, c->stream));
     for (uint64_t at = 0; at < n_points; at += CH) {
       const uint64_t n = std::min(CH, n_points - at);
-      CU(c, cudaMemcpyAsync(stage, points + at, n * sizeof(mm_ipoint), cudaMemcpyHostToDevice, c->stream));
-      CU(c, mm_upload_pack_points((const mm_ipoint *)stage, n, n_contigs, (uint64_t *)(c->blob + h.off_pts) + at, d_err, c->stream));
+      CU(c, cudaMemcpyAsync(stage.p, points + at, n * sizeof(mm_ipoint), cudaMemcpyHostToDevice, c->stream));
+      CU(c, mm_upload_pack_points((const mm_ipoint *)stage.p, n, n_contigs, (uint64_t *)(c->blob + h.off_pts) + at, d_err.p, c->stream));
       CU(c, cudaStreamSynchronize(c->stream));
     }
-    cudaFree(stage_buf.p); stage_buf.p = nullptr;
+    stage.release();
     /* open-addressing table, filled on the device */
     CU(c, cudaMemsetAsync(c->blob + h.off_tab, 0, tab_slots * sizeof(mm_tab_slot), c->stream));
     if (n_keys) {
-      dev_tmp keys_buf, offs_buf, freq_buf;
-      CU(c, cudaMalloc(&keys_buf.p, n_keys * 8));
-      CU(c, cudaMalloc(&offs_buf.p, (n_keys + 1) * 8));
-      CU(c, cudaMalloc(&freq_buf.p, n_keys));
-      uint64_t *d_keys = (uint64_t *)keys_buf.p, *d_offs = (uint64_t *)offs_buf.p;
-      uint8_t *d_freq = (uint8_t *)freq_buf.p;
-      CU(c, cudaMemcpyAsync(d_keys, keys, n_keys * 8, cudaMemcpyHostToDevice, c->stream));
-      CU(c, cudaMemcpyAsync(d_offs, offsets, (n_keys + 1) * 8, cudaMemcpyHostToDevice, c->stream));
-      CU(c, cudaMemcpyAsync(d_freq, key_is_freq, n_keys, cudaMemcpyHostToDevice, c->stream));
-      CU(c, mm_upload_build_table(d_keys, d_offs, d_freq, n_keys, (mm_tab_slot *)(c->blob + h.off_tab), tab_log2, d_err, c->stream));
+      dev_array<uint64_t> d_keys, d_offs;
+      dev_array<uint8_t> d_freq;
+      if ((rc = d_keys.reserve(c, n_keys, n_keys)) || (rc = d_offs.reserve(c, n_keys + 1, n_keys + 1)) ||
+          (rc = d_freq.reserve(c, n_keys, n_keys)))
+        return rc;
+      CU(c, cudaMemcpyAsync(d_keys.p, keys, n_keys * 8, cudaMemcpyHostToDevice, c->stream));
+      CU(c, cudaMemcpyAsync(d_offs.p, offsets, (n_keys + 1) * 8, cudaMemcpyHostToDevice, c->stream));
+      CU(c, cudaMemcpyAsync(d_freq.p, key_is_freq, n_keys, cudaMemcpyHostToDevice, c->stream));
+      CU(c, mm_upload_build_table(d_keys.p, d_offs.p, d_freq.p, n_keys, (mm_tab_slot *)(c->blob + h.off_tab), h.tab_log2, d_err.p, c->stream));
       CU(c, cudaStreamSynchronize(c->stream));
     }
     uint32_t err = 0;
-    CU(c, cudaMemcpyAsync(&err, d_err, 4, cudaMemcpyDeviceToHost, c->stream));
+    CU(c, cudaMemcpyAsync(&err, d_err.p, 4, cudaMemcpyDeviceToHost, c->stream));
     CU(c, cudaStreamSynchronize(c->stream));
     if (err & 1) return fail(c, MM_EINVAL, "an interval point has a bad seqId or a negative position");
     if (err & 2) return fail(c, MM_EINVAL, "a key has no or too many (>= 2^24) interval points, or offsets overflow");
     if (err & 4) return fail(c, MM_EINVAL, "duplicate key in the lookup index");
   }
-  CU(c, cudaMemcpyAsync(c->blob + h.off_contig_len, contig_len, (size_t)n_contigs * 4, cudaMemcpyHostToDevice, c->stream));
-  std::vector<int32_t> tmp((size_t)n_contigs, -1);
-  CU(c, cudaMemcpyAsync(c->blob + h.off_contig_name_id, contig_name_id ? contig_name_id : tmp.data(), (size_t)n_contigs * 4, cudaMemcpyHostToDevice, c->stream));
-  CU(c, cudaStreamSynchronize(c->stream)); /* tmp is rewritten below */
-  std::fill(tmp.begin(), tmp.end(), 0);
-  CU(c, cudaMemcpyAsync(c->blob + h.off_contig_group, contig_group ? contig_group : tmp.data(), (size_t)n_contigs * 4, cudaMemcpyHostToDevice, c->stream));
-  CU(c, cudaMemcpyAsync(c->blob, &c->hdr, sizeof(c->hdr), cudaMemcpyHostToDevice, c->stream));
-  CU(c, cudaStreamSynchronize(c->stream));
-  resolve_index(c);
-  c->blob_ready = true;
-  guard.done = true;
-  return write_tables(c);
+  return finish_blob(c, contig_len, contig_name_id, contig_group);
 }
 
 int mm_tables_upload(mm_ctx *c, const int32_t *cut, int32_t n_cut, const int32_t *mh, int32_t n_mh)
@@ -818,10 +815,9 @@ int mm_index_blob_alloc(mm_ctx *c, uint64_t n_bytes, void **blob)
 {
   if (!c || !blob || n_bytes < sizeof(mm_blob_header)) return MM_EINVAL;
   CU(c, cudaSetDevice(c->device));
-  if (c->blob && c->blob_owned) cudaFree(c->blob);
-  c->blob = nullptr; c->blob_ready = false;
-  CU(c, cudaMalloc((void **)&c->blob, n_bytes));
-  c->blob_bytes = n_bytes; c->blob_owned = true; c->share_src = nullptr;
+  mm_blob_header h{}; /* the real one arrives with the image (mm_index_adopt_blob) */
+  h.total_bytes = n_bytes;
+  if (int rc = replace_blob(c, h)) return rc;
   *blob = c->blob;
   return MM_OK;
 }
@@ -843,7 +839,7 @@ int mm_ctx_share_index(mm_ctx *c, const mm_ctx *src)
   if (!c || !src) return MM_EINVAL;
   if (!src->blob_ready) return fail(c, MM_ESTATE, "source context has no index");
   if (c->device != src->device) return fail(c, MM_EINVAL, "contexts are on different devices");
-  if (c->blob && c->blob_owned) { cudaSetDevice(c->device); cudaFree(c->blob); }
+  release_blob(c);
   c->blob = src->blob; c->blob_bytes = src->blob_bytes; c->blob_owned = false;
   c->hdr = src->hdr;
   c->cutoffs = src->cutoffs; c->min_hits = src->min_hits;
@@ -859,7 +855,7 @@ static int batch_upload_any(mm_ctx *c, const void *bases, uint64_t n_bases, cons
   int rc = upload_batch(c, bases, n_bases, segs, n_segs, packed);
   if (rc) return rc;
   CU(c, wait_stream(c));
-  cudaEventElapsedTime(&c->stage_ms[3], c->ev[6], c->ev[7]);
+  cudaEventElapsedTime(&c->stage_ms[3], c->ev[EV_H2D_BEGIN], c->ev[EV_H2D_END]);
   return MM_OK;
 }
 int mm_batch_upload(mm_ctx *c, const char *bases, uint64_t n_bases, const mm_segment *segs, uint64_t n_segs)
@@ -887,13 +883,13 @@ int mm_batch_fetch(mm_ctx *c, mm_segment_result *seg_results, mm_l1_candidate *c
   if (!c || !c->batch_mapped) return fail(c, MM_ESTATE, "no mapped batch");
   if (cand_cap < c->n_cands || loci_cap < c->n_loci) return fail(c, MM_ECAPACITY, "output capacity too small");
   CU(c, cudaSetDevice(c->device));
-  CU(c, cudaEventRecord(c->ev[5], c->stream));
-  if (seg_results) CU(c, cudaMemcpyAsync(seg_results, c->d_seg_res, c->n_segs * sizeof(mm_segment_result), cudaMemcpyDeviceToHost, c->stream));
-  if (cands && c->n_cands) CU(c, cudaMemcpyAsync(cands, c->d_cands, c->n_cands * sizeof(mm_l1_candidate), cudaMemcpyDeviceToHost, c->stream));
-  if (loci && c->n_loci) CU(c, cudaMemcpyAsync(loci, c->d_loci, c->n_loci * sizeof(mm_l2_locus), cudaMemcpyDeviceToHost, c->stream));
-  CU(c, cudaEventRecord(c->ev[6], c->stream));
+  CU(c, cudaEventRecord(c->ev[EV_D2H_BEGIN], c->stream));
+  if (seg_results) CU(c, cudaMemcpyAsync(seg_results, c->d_seg_res.p, c->n_segs * sizeof(mm_segment_result), cudaMemcpyDeviceToHost, c->stream));
+  if (cands && c->n_cands) CU(c, cudaMemcpyAsync(cands, c->d_cands.p, c->n_cands * sizeof(mm_l1_candidate), cudaMemcpyDeviceToHost, c->stream));
+  if (loci && c->n_loci) CU(c, cudaMemcpyAsync(loci, c->d_loci.p, c->n_loci * sizeof(mm_l2_locus), cudaMemcpyDeviceToHost, c->stream));
+  CU(c, cudaEventRecord(c->ev[EV_D2H_END], c->stream));
   CU(c, wait_stream(c));
-  cudaEventElapsedTime(&c->stage_ms[4], c->ev[5], c->ev[6]);
+  cudaEventElapsedTime(&c->stage_ms[4], c->ev[EV_D2H_BEGIN], c->ev[EV_D2H_END]);
   return MM_OK;
 }
 
@@ -907,11 +903,11 @@ int mm_batch_fetch_sketch(mm_ctx *c, mm_minmer *out, int32_t *out_count)
   std::vector<int8_t> ss(n);
   std::vector<mm_segment_result> sr(c->n_segs);
   std::vector<mm_segment> sg(c->n_segs);
-  CU(c, cudaMemcpyAsync(hh.data(), c->d_sk_hash, n * 8, cudaMemcpyDeviceToHost, c->stream));
-  CU(c, cudaMemcpyAsync(pp.data(), c->d_sk_pos, n * 8, cudaMemcpyDeviceToHost, c->stream));
-  CU(c, cudaMemcpyAsync(ss.data(), c->d_sk_strand, n, cudaMemcpyDeviceToHost, c->stream));
-  CU(c, cudaMemcpyAsync(sr.data(), c->d_seg_res, c->n_segs * sizeof(mm_segment_result), cudaMemcpyDeviceToHost, c->stream));
-  CU(c, cudaMemcpyAsync(sg.data(), c->d_segs, c->n_segs * sizeof(mm_segment), cudaMemcpyDeviceToHost, c->stream));
+  CU(c, cudaMemcpyAsync(hh.data(), c->d_sk_hash.p, n * 8, cudaMemcpyDeviceToHost, c->stream));
+  CU(c, cudaMemcpyAsync(pp.data(), c->d_sk_pos.p, n * 8, cudaMemcpyDeviceToHost, c->stream));
+  CU(c, cudaMemcpyAsync(ss.data(), c->d_sk_strand.p, n, cudaMemcpyDeviceToHost, c->stream));
+  CU(c, cudaMemcpyAsync(sr.data(), c->d_seg_res.p, c->n_segs * sizeof(mm_segment_result), cudaMemcpyDeviceToHost, c->stream));
+  CU(c, cudaMemcpyAsync(sg.data(), c->d_segs.p, c->n_segs * sizeof(mm_segment), cudaMemcpyDeviceToHost, c->stream));
   CU(c, cudaStreamSynchronize(c->stream));
   for (uint64_t s = 0; s < c->n_segs; s++) {
     out_count[s] = sr[s].sketch_size;
@@ -932,16 +928,16 @@ int mm_sketch_segments(mm_ctx *c, const char *bases, uint64_t n_bases, const mm_
   if (rc) return rc;
   mm_dev_batch b = make_batch(c);
   if ((rc = launch_pack_if_ascii(c))) return rc;
-  ZERO_WORDS(c, c->d_counters, 16);
-  CU(c, cudaEventRecord(c->ev[0], c->stream));
+  ZERO_WORDS(c, c->d_counters.p, 16);
+  CU(c, cudaEventRecord(c->ev[EV_K1_BEGIN], c->stream));
   CU(c, mm_launch_sketch(c->params, b, c->stream, c->sm_count, c->sk_mode));
-  CU(c, cudaEventRecord(c->ev[1], c->stream));
+  CU(c, cudaEventRecord(c->ev[EV_K1_END], c->stream));
   c->launches += c->sk_mode ? 1 : 2;
   CU(c, cudaStreamSynchronize(c->stream));
-  cudaEventElapsedTime(&c->stage_ms[0], c->ev[0], c->ev[1]);
+  cudaEventElapsedTime(&c->stage_ms[0], c->ev[EV_K1_BEGIN], c->ev[EV_K1_END]);
   {
     uint32_t h9 = 0;
-    if (cudaMemcpy(&h9, c->d_counters + 9, 4, cudaMemcpyDeviceToHost) == cudaSuccess) c->diag[MM_DIAG_SKETCH_GENERAL_SEGMENTS] += h9;
+    if (cudaMemcpy(&h9, c->d_counters.p + 9, 4, cudaMemcpyDeviceToHost) == cudaSuccess) c->diag[MM_DIAG_SKETCH_GENERAL_SEGMENTS] += h9;
   }
   c->batch_mapped = true; /* sketches only; fetch_sketch reads sketch_size == raw count */
   rc = mm_batch_fetch_sketch(c, out, out_count);
@@ -957,7 +953,7 @@ static int map_segments_any(mm_ctx *c, const void *bases, uint64_t n_bases, cons
   int rc = upload_batch(c, bases, n_bases, segs, n_segs, packed);
   if (rc) return rc;
   if ((rc = run_pipeline(c))) return rc;
-  cudaEventElapsedTime(&c->stage_ms[3], c->ev[6], c->ev[7]);
+  cudaEventElapsedTime(&c->stage_ms[3], c->ev[EV_H2D_BEGIN], c->ev[EV_H2D_END]);
   *n_candidates = c->n_cands;
   *n_loci = c->n_loci;
   if (cand_cap < c->n_cands || loci_cap < c->n_loci) return fail(c, MM_ECAPACITY, "need %llu candidates, %llu loci", (unsigned long long)c->n_cands, (unsigned long long)c->n_loci);
@@ -1051,66 +1047,48 @@ int mm_index_build(mm_ctx *c, const char *seqs, int seqs_on_device, const uint64
   if (n_contigs < 1 || !contig_offsets || !seqs) return fail(c, MM_EINVAL, "no contigs");
   CU(c, cudaSetDevice(c->device));
   const auto t0 = std::chrono::steady_clock::now();
-  if (c->blob && c->blob_owned) { cudaFree(c->blob); }
-  c->blob = nullptr; c->blob_ready = false;
+  release_blob(c);
   mm_built_index_free(&c->built);
   c->built_kept = false;
-  const uint64_t total = contig_offsets[n_contigs];
-  uint8_t *d_seq = (uint8_t *)seqs;
-  uint8_t *staged = nullptr;
-  if (!seqs_on_device) {
-    CU(c, cudaMalloc((void **)&staged, total + 64));
-    CU(c, cudaMemcpyAsync(staged, seqs, total, cudaMemcpyHostToDevice, c->stream));
-    d_seq = staged;
+  /* every early return below releases the temporaries: the staged text, the builder's arrays, the counters */
+  struct built_guard {
+    mm_built_index b;
+    ~built_guard() { mm_built_index_free(&b); }
+  } built;
+  mm_built_index &B = built.b;
+  int rc;
+  {
+    const uint64_t total = contig_offsets[n_contigs];
+    const uint8_t *d_seq = (const uint8_t *)seqs;
+    dev_array<uint8_t> staged;
+    if (!seqs_on_device) {
+      if ((rc = staged.reserve(c, total + 64, total + 64))) return rc;
+      CU(c, cudaMemcpyAsync(staged.p, seqs, total, cudaMemcpyHostToDevice, c->stream));
+      d_seq = staged.p;
+    }
+    std::string err;
+    rc = mm_build_index_device(c->params, d_seq, contig_offsets, n_contigs, kmer_pct_threshold, c->stream, c->sm_count, &B, err);
+    if (rc != MM_OK) return fail(c, rc, "index build: %s", err.c_str());
   }
-  mm_built_index B;
-  std::string err;
-  int rc = mm_build_index_device(c->params, d_seq, contig_offsets, n_contigs, kmer_pct_threshold, c->stream, c->sm_count, &B, err);
-  if (staged) cudaFree(staged);
-  if (rc != MM_OK) { mm_built_index_free(&B); return fail(c, rc, "index build: %s", err.c_str()); }
   c->launches += 12;
 
   const uint64_t n_mi = B.n_minmers, n_keys = B.n_keys, n_points = B.n_points;
-  if (n_mi >= (1ULL << 32)) { mm_built_index_free(&B); return fail(c, MM_EINVAL, "more than 2^32 minmers"); }
+  if (n_mi >= (1ULL << 32)) return fail(c, MM_EINVAL, "more than 2^32 minmers");
   /* contig_start from the seqId column */
   std::vector<uint64_t> cstart((size_t)n_contigs + 1, 0);
   if (n_mi) {
-    unsigned long long *d_cnt = nullptr;
-    CU(c, cudaMalloc((void **)&d_cnt, ((size_t)n_contigs + 1) * 8));
-    CU(c, cudaMemsetAsync(d_cnt, 0, ((size_t)n_contigs + 1) * 8, c->stream));
-    k_count_seq<<<(uint32_t)((n_mi + 255) / 256), 256, 0, c->stream>>>(n_mi, B.seq, d_cnt);
+    dev_array<unsigned long long> d_cnt;
+    if ((rc = d_cnt.reserve(c, (size_t)n_contigs + 1, (size_t)n_contigs + 1))) return rc;
+    CU(c, cudaMemsetAsync(d_cnt.p, 0, ((size_t)n_contigs + 1) * 8, c->stream));
+    k_count_seq<<<(uint32_t)((n_mi + 255) / 256), 256, 0, c->stream>>>(n_mi, B.seq, d_cnt.p);
     std::vector<unsigned long long> cnt((size_t)n_contigs + 1);
-    CU(c, cudaMemcpyAsync(cnt.data(), d_cnt, ((size_t)n_contigs + 1) * 8, cudaMemcpyDeviceToHost, c->stream));
+    CU(c, cudaMemcpyAsync(cnt.data(), d_cnt.p, ((size_t)n_contigs + 1) * 8, cudaMemcpyDeviceToHost, c->stream));
     CU(c, cudaStreamSynchronize(c->stream));
-    cudaFree(d_cnt);
     for (int32_t q = 0; q < n_contigs; q++) cstart[(size_t)q + 1] = cstart[(size_t)q] + cnt[(size_t)q];
   }
-  int tab_log2 = 4;
-  while ((1ULL << tab_log2) < 2 * n_keys + 2) tab_log2++;
-  const uint64_t tab_slots = 1ULL << tab_log2;
-  mm_blob_header h{};
-  h.magic = MM_BLOB_MAGIC;
-  h.n_minmers = n_mi; h.n_keys = n_keys; h.n_points = n_points;
-  h.n_contigs = n_contigs; h.tab_log2 = tab_log2;
-  uint64_t o = align_up(sizeof(mm_blob_header), 256);
-  auto place = [&](uint64_t bytes) { uint64_t at = o; o = align_up(o + bytes, 256); return at; };
-  h.off_idx_hash = place((n_mi + 1) * 8);
-  h.off_idx_wpos = place((n_mi + 1) * 4);
-  h.off_idx_wend = place((n_mi + 1) * 4);
-  h.off_idx_strand = place(n_mi + 1);
-  h.off_contig_start = place(((uint64_t)n_contigs + 1) * 8);
-  h.off_idx2_hash = place((n_mi + 1) * 8);
-  h.off_idx2_wend = place((n_mi + 1) * 4);
-  h.off_tab = place(tab_slots * sizeof(mm_tab_slot));
-  h.off_pts = place((n_points + 1) * 8);
-  h.off_contig_len = place((uint64_t)n_contigs * 4);
-  h.off_contig_name_id = place((uint64_t)n_contigs * 4);
-  h.off_contig_group = place((uint64_t)n_contigs * 4);
-  h.off_cutoffs = place(TABLE_REGION_BYTES);
-  h.off_min_hits = place(TABLE_REGION_BYTES);
-  h.total_bytes = o;
-  if (cudaMalloc((void **)&c->blob, o) != cudaSuccess) { cudaGetLastError(); mm_built_index_free(&B); return fail(c, MM_ENOMEM, "cannot allocate the index image (%llu bytes)", (unsigned long long)o); }
-  c->blob_bytes = o; c->blob_owned = true; c->hdr = h; c->share_src = nullptr;
+  const mm_blob_header h = blob_layout(n_mi, n_keys, n_points, n_contigs);
+  if ((rc = replace_blob(c, h))) return rc;
+  blob_guard guard{c};
   if (n_mi) {
     CU(c, cudaMemcpyAsync(c->blob + h.off_idx_hash, B.hash, n_mi * 8, cudaMemcpyDeviceToDevice, c->stream));
     CU(c, cudaMemcpyAsync(c->blob + h.off_idx_wpos, B.wpos, n_mi * 4, cudaMemcpyDeviceToDevice, c->stream));
@@ -1125,29 +1103,20 @@ int mm_index_build(mm_ctx *c, const char *seqs, int seqs_on_device, const uint64
                              (const uint64_t *)(c->blob + h.off_contig_start), n_contigs, n_mi,
                              (uint64_t *)(c->blob + h.off_idx2_hash), (int32_t *)(c->blob + h.off_idx2_wend), c->stream));
   if (n_points) CU(c, cudaMemcpyAsync(c->blob + h.off_pts, B.pts, n_points * 8, cudaMemcpyDeviceToDevice, c->stream));
-  CU(c, cudaMemsetAsync(c->blob + h.off_tab, 0, tab_slots * sizeof(mm_tab_slot), c->stream));
+  CU(c, cudaMemsetAsync(c->blob + h.off_tab, 0, (1ULL << h.tab_log2) * sizeof(mm_tab_slot), c->stream));
   if (n_keys) {
-    uint32_t *d_err = nullptr;
-    CU(c, cudaMalloc((void **)&d_err, 4));
-    CU(c, cudaMemsetAsync(d_err, 0, 4, c->stream));
-    CU(c, mm_upload_build_table(B.keys, B.offs, B.is_freq, n_keys, (mm_tab_slot *)(c->blob + h.off_tab), tab_log2, d_err, c->stream));
+    dev_array<uint32_t> d_err;
+    if ((rc = d_err.reserve(c, 1, 1))) return rc;
+    CU(c, cudaMemsetAsync(d_err.p, 0, 4, c->stream));
+    CU(c, mm_upload_build_table(B.keys, B.offs, B.is_freq, n_keys, (mm_tab_slot *)(c->blob + h.off_tab), h.tab_log2, d_err.p, c->stream));
     uint32_t e = 0;
-    CU(c, cudaMemcpyAsync(&e, d_err, 4, cudaMemcpyDeviceToHost, c->stream));
+    CU(c, cudaMemcpyAsync(&e, d_err.p, 4, cudaMemcpyDeviceToHost, c->stream));
     CU(c, cudaStreamSynchronize(c->stream));
-    cudaFree(d_err);
-    if (e) { mm_built_index_free(&B); return fail(c, MM_EINVAL, "lookup table build failed (code %u)", e); }
+    if (e) return fail(c, MM_EINVAL, "lookup table build failed (code %u)", e);
   }
-  std::vector<int32_t> clen((size_t)n_contigs), tmp((size_t)n_contigs, -1);
+  std::vector<int32_t> clen((size_t)n_contigs);
   for (int32_t q = 0; q < n_contigs; q++) clen[(size_t)q] = (int32_t)(contig_offsets[q + 1] - contig_offsets[q]);
-  CU(c, cudaMemcpyAsync(c->blob + h.off_contig_len, clen.data(), (size_t)n_contigs * 4, cudaMemcpyHostToDevice, c->stream));
-  CU(c, cudaMemcpyAsync(c->blob + h.off_contig_name_id, contig_name_id ? contig_name_id : tmp.data(), (size_t)n_contigs * 4, cudaMemcpyHostToDevice, c->stream));
-  CU(c, cudaStreamSynchronize(c->stream));
-  std::fill(tmp.begin(), tmp.end(), 0);
-  CU(c, cudaMemcpyAsync(c->blob + h.off_contig_group, contig_group ? contig_group : tmp.data(), (size_t)n_contigs * 4, cudaMemcpyHostToDevice, c->stream));
-  CU(c, cudaMemcpyAsync(c->blob, &c->hdr, sizeof(c->hdr), cudaMemcpyHostToDevice, c->stream));
-  CU(c, cudaStreamSynchronize(c->stream));
-  resolve_index(c);
-  c->blob_ready = true;
+  if ((rc = finish_blob(c, clen.data(), contig_name_id, contig_group))) return rc;
   if (stats) {
     memset(stats, 0, sizeof *stats);
     stats->n_minmers = n_mi; stats->n_minmers_before_filter = B.n_minmers_before_filter; stats->n_keys = n_keys; stats->n_points = n_points;
@@ -1156,9 +1125,12 @@ int mm_index_build(mm_ctx *c, const char *seqs, int seqs_on_device, const uint64
     stats->hist_max_keys = B.hist_max_keys; stats->ms_scan = B.ms_scan; stats->ms_post = B.ms_post; stats->ms_lookup = B.ms_lookup;
     stats->ms_total = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
   }
-  if (keep_lookup) { c->built = B; c->built_kept = true; }
-  else mm_built_index_free(&B);
-  return write_tables(c);
+  if (keep_lookup) {
+    c->built = B;
+    c->built_kept = true;
+    B = mm_built_index{};
+  }
+  return MM_OK;
 }
 
 /* host copies of what mm_index_build left on the device (needs keep_lookup); any output may be NULL */
@@ -1189,12 +1161,11 @@ int mm_index_download(mm_ctx *c, mm_minmer *mi, uint64_t *keys, uint64_t *offset
   if (offsets) CU(c, cudaMemcpy(offsets, B.offs, (B.n_keys + 1) * 8, cudaMemcpyDeviceToHost));
   if (is_freq && B.n_keys) CU(c, cudaMemcpy(is_freq, B.is_freq, B.n_keys, cudaMemcpyDeviceToHost));
   if (points && B.n_points) {
-    mm_ipoint *d = nullptr;
-    CU(c, cudaMalloc((void **)&d, B.n_points * sizeof(mm_ipoint)));
-    k_unpack_points<<<(uint32_t)((B.n_points + 255) / 256), 256, 0, c->stream>>>(B.n_points, (const uint64_t *)(c->blob + h.off_pts), B.keys, B.offs, B.n_keys, d);
-    CU(c, cudaMemcpyAsync(points, d, B.n_points * sizeof(mm_ipoint), cudaMemcpyDeviceToHost, c->stream));
+    dev_array<mm_ipoint> d;
+    if (int rc = d.reserve(c, B.n_points, B.n_points)) return rc;
+    k_unpack_points<<<(uint32_t)((B.n_points + 255) / 256), 256, 0, c->stream>>>(B.n_points, (const uint64_t *)(c->blob + h.off_pts), B.keys, B.offs, B.n_keys, d.p);
+    CU(c, cudaMemcpyAsync(points, d.p, B.n_points * sizeof(mm_ipoint), cudaMemcpyDeviceToHost, c->stream));
     CU(c, cudaStreamSynchronize(c->stream));
-    cudaFree(d);
   }
   return MM_OK;
 }

@@ -1,6 +1,6 @@
 #!/bin/bash
-# e2e pipeline experiments on a reduced workload (400k reads vs 300 Mbp): per-part kernel times (MM_TRACE) with the
-# copy engine upload, without uploads, and with the SM-driven upload kernel.
+# e2e pipeline experiments on a reduced workload (400k reads vs 300 Mbp): per-part kernel times (MM_TRACE) under
+# different host thread counts, wait modes and host-library switches.
 W="--config 2 --reads 400000 --ref-bp 300000000 --contigs 32 --sketch 220 --no-cpu-baseline --steps 2 --warmup 2"
 run() { # name, env...
   local name=$1; shift
@@ -27,12 +27,10 @@ for v in "$@"; do
     few2spin) run few2spin BENCH_HOST_THREADS=2 MM_BLOCKING_WAIT=0 ;;
     few4) run few4 BENCH_HOST_THREADS=4 ;;
     noramp) run noramp MM_NO_RAMP=1 ;;
-    skip) run skip MM_SKIP_H2D=12 ;;
     serial) run serial MM_LANES=1 ;;
     tail1) run tail1 MM_TAIL_THREADS=1 ;;
     tail6) run tail6 MM_TAIL_THREADS=6 ;;
     nogate) run nogate MM_NO_GATE=1 ;;
-    kern8) run kern8 MM_UPLOAD_KERNEL=8 ;;
     block) run block MM_BLOCKING_WAIT=1 ;;
   esac
 done
